@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the env-step hot path (BASELINE.json metric: env-steps/s and agent-steps/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1] ("c2"): flight_easy 3a15t AM0TM0, 4096 envs per kernel launch.
 4096 envs are ~2.6 MB of state+outputs, i.e. L2-resident, so the bench keeps 64 independent 4096-env batches
@@ -137,7 +137,11 @@ class ClockSampler:
 # ----------------------------------------------------------------------------------------------------------------
 def reference_kind():
     from oracle import refharness as rh
-    return "reference" if rh.reference_available() else "port"
+    if rh.reference_available():
+        return "reference"
+    print("bench.py: no reference checkout (COOPSEARCH_REFERENCE, BASELINE.json reference_path) and no staged oracle/_ref: "
+          "the CPU baseline times the Python oracle port instead of the reference's own code", file=sys.stderr)
+    return "port"
 
 
 def _make_ref_env(kind, n, am):
@@ -371,14 +375,39 @@ def silence(fn, *a, **k):
         return fn(*a, **k)
 
 
-MIN_TIMED_MS = 60.0       # the timed region is repeated until it is at least this long; the median repetition is reported
+MIN_TIMED_MS = 60.0       # the host-buffer (e2e) blocks are repeated until they last at least this long
+DUMP_BYTES = 60 << 20     # --dump-outputs data: with the .npy headers under 64 MB (64e6 bytes) in all
+SPREAD_REPLAYS = 5        # untimed replays after the timed one whose min / max show how much one replay varies
 
 
-def run_gpu_workload(cs, torch, name, steps, warmup, device, rank, world, want_e2e=True, burn_in_s=0.3):
-    """One workload on this rank.  The `steps` bench steps are captured into ONE CUDA graph; the timed region replays
-    that graph R times back to back (R such that the region lasts >= MIN_TIMED_MS), every replay bracketed by CUDA
-    events on the launching stream, and the MEDIAN replay is reported: `steps` steps of a 60 us kernel are 1.4 ms,
-    which measures launch jitter, not the kernel."""
+def dump_outputs(torch, envs, kind, directory):
+    """Writes what the last step left in the env buffers -- reward, terminated, win (flight), target_find, get_obs(),
+    get_state() and, for search, the action masks -- as <directory>/<name>.npy in float32, one row per env in global env
+    id order.  When all rows would exceed DUMP_BYTES, every array keeps the same fixed, seeded sample of env rows."""
+    cat = lambda get: torch.cat([get(e).float() for e in envs])
+    arrays = {"reward": cat(lambda e: e._reward), "terminated": cat(lambda e: e._terminated)}
+    if kind != "search":
+        arrays["win"] = cat(lambda e: e.win_flag)
+    arrays.update(target_find=cat(lambda e: e.target_find), obs=cat(lambda e: e.get_obs()), state=cat(lambda e: e.get_state()))
+    if kind == "search":
+        arrays["avail"] = cat(lambda e: e.get_avail_actions())
+    rows = arrays["reward"].shape[0]
+    row_bytes = sum(4 * a[0].numel() for a in arrays.values())
+    if rows * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(rows, DUMP_BYTES // row_bytes, replace=False))
+        idx = torch.from_numpy(keep).to(arrays["reward"].device)
+        arrays = {k: a.index_select(0, idx) for k, a in arrays.items()}
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a.cpu().numpy())
+
+
+def run_gpu_workload(cs, torch, name, steps, warmup, device, rank, world, want_e2e=True, burn_in_steps=6000, dump_dir=None):
+    """One workload on this rank.  The `steps` bench steps are captured into ONE CUDA graph; the timed region is one
+    replay of it, bracketed by CUDA events on the launching stream.  Before it, untimed: `warmup` steps, then
+    `burn_in_steps` rounded up to whole replays, queued back to back so that clocks have ramped under this load and
+    the timed replay starts while the GPU is still busy (no launch gap in the region).  Every count is fixed, so the
+    same arguments step the envs through the same sequence; `dump_dir` receives what the last timed step computed."""
     w = WORKLOADS[name]
     n = w["n"]
     A = 4 if w["kind"] == "search" else 3
@@ -439,46 +468,39 @@ def run_gpu_workload(cs, torch, name, steps, warmup, device, rank, world, want_e
             for k in range(steps):
                 one_step(k)
             join_maps()
-    torch.cuda.synchronize(device)
-
-    # clock burn-in + warm-up: the same work, untimed, so that the sampler sees the GPU under THIS load and clocks have ramped
-    t_end = time.perf_counter() + burn_in_s
-    with torch.cuda.stream(side):
-        gsteps.replay()
-        torch.cuda.synchronize(device)
-        t0 = time.perf_counter()
-        gsteps.replay()
-        torch.cuda.synchronize(device)
-        est_ms = 1000.0 * (time.perf_counter() - t0)
-        while time.perf_counter() < t_end:
-            gsteps.replay()
-            torch.cuda.synchronize(device)
-        for k in range(warmup):                                # W warm-up steps (already far exceeded by the burn-in)
+        for k in range(warmup):
             one_step(k)
         join_maps()
     torch.cuda.synchronize(device)
-    reps = int(min(4000, max(1, -(-MIN_TIMED_MS // max(est_ms, 1e-3)))))
     if world > 1:
-        reps_t = torch.tensor([reps], device=device)
-        torch.distributed.all_reduce(reps_t, op=torch.distributed.ReduceOp.MAX)     # the same replay count on every rank
-        reps = int(reps_t.item())
         torch.distributed.barrier()
+    burn_in_replays = -(-burn_in_steps // steps)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    with torch.cuda.stream(side):
+        for _ in range(burn_in_replays):
+            gsteps.replay()
+        e0.record()
+        gsteps.replay()                                        # the timed region: exactly `steps` steps
+        e1.record()
     torch.cuda.synchronize(device)
-    evs = [torch.cuda.Event(enable_timing=True) for _ in range(reps + 1)]
+    if world > 1:
+        torch.distributed.barrier()
+    ms = e0.elapsed_time(e1)
+    if dump_dir is not None:
+        dump_outputs(torch, envs, w["kind"], dump_dir)
+    # noise check, not part of the timed figure: SPREAD_REPLAYS more replays of the same graph, each bracketed by events
+    evs = [torch.cuda.Event(enable_timing=True) for _ in range(SPREAD_REPLAYS + 1)]
     with torch.cuda.stream(side):
         evs[0].record()
-        for r in range(reps):
+        for r in range(SPREAD_REPLAYS):
             gsteps.replay()
             evs[r + 1].record()
     torch.cuda.synchronize(device)
-    if world > 1:
-        torch.distributed.barrier()
-    rep_ms = sorted(evs[r].elapsed_time(evs[r + 1]) for r in range(reps))
-    ms = rep_ms[len(rep_ms) // 2]                              # median replay of exactly `steps` steps
+    spread = [evs[r].elapsed_time(evs[r + 1]) for r in range(SPREAD_REPLAYS)]
     launches = steps * (1 if grouped is not None else len(envs))
     env_count = sum(e.num_envs for e in envs)
     out = dict(grouped=grouped is not None, ms_total=ms, ms_per_step=ms / steps, env_steps_per_step=env_count, launches=launches, streams=nstreams,
-               kernels=kernels_per_step * steps, timed_reps=reps, timed_region_ms=evs[0].elapsed_time(evs[reps]), ms_min=rep_ms[0], ms_max=rep_ms[-1],
+               kernels=kernels_per_step * steps, burn_in_steps=burn_in_replays * steps, check_replays_ms=[min(spread), max(spread)],
                us_per_launch=1000.0 * ms / launches, lanes_per_env=getattr(envs[0], "lanes_per_env", None),
                envs_per_launch=env_count if grouped is not None else envs[0].num_envs)
 
@@ -730,7 +752,7 @@ def measure_c1(cs, torch, device, seconds=4.0):
     E=1 SingleEnvAdapter (one kernel launch per call: the latency floor of the drop-in, not a throughput figure)."""
     from oracle import refharness as rh
     if not rh.reference_available():
-        return {"unavailable": "oracle/_ref is not staged on this box (run __graft_entry__.build() where /root/reference exists)"}
+        return {"unavailable": "no reference checkout (COOPSEARCH_REFERENCE, BASELINE.json reference_path) and no staged oracle/_ref"}
     ref = rh.import_reference()
     circle = rh.load_targets_reference_semantics(os.path.join(rh.REFERENCE_ROOT, "flight_targets.txt"))
     v_ref, eps, steps, found = rollout_worker_throughput(lambda a: rh.quiet(ref["FlightSearchEnvEasy"], a, circle), 1, seconds)
@@ -789,8 +811,9 @@ def config_for(name, world):
         "actions": "uniform-random policy: pre-generated u8 tensors resident in HBM (flight) / drawn in-kernel with Philox (search, shard-invariance runs)",
         "launch": "the --steps bench steps are captured into one CUDA graph; one step = " +
                   ("ONE grouped launch that steps every handle (cs_flight_group_step)" if grouped else "one launch per handle"),
-        "timing": "the K-step graph is replayed back to back until the timed region is >= %d ms; every replay is bracketed by CUDA events on the launching stream; "
-                  "the median replay / K is ms_per_step (max over ranks); barrier + synchronize on both sides of the region" % MIN_TIMED_MS,
+        "timing": "the timed region is one replay of the K-step graph, bracketed by CUDA events on the launching stream and queued behind the untimed "
+                  "burn-in replays; its duration / K is ms_per_step (max over ranks); synchronize + barrier before the burn-in and after the region; "
+                  "%d more replays after it, untimed for the result, give timed.check_replays_ms_min_max (raise --steps where they spread)" % SPREAD_REPLAYS,
         "l2": "working set of all batches exceeds the 126 MB L2; batches are revisited round-robin, no flush",
         "parallelism": "dp%d (env instances sharded by global id, no data-path collective)" % world,
     }
@@ -840,7 +863,8 @@ def extra_entry(cs, torch, name, r, peak, device, with_touched=True):
     v = r["env_steps_per_step"] / (r["ms_per_step"] / 1000.0)
     gbs = pu * r["envs_per_launch"] / (1e-6 * r["us_per_launch"]) / 1e9
     out = {"workload": ww["desc"], "kernel": kernel_name(ww, r["lanes_per_env"], r["grouped"]), "value": v, "unit": "env-steps/s",
-           "agent_steps_per_s": v * ww["n"], "us_per_launch": r["us_per_launch"], "timed_reps": r["timed_reps"], "timed_region_ms": r["timed_region_ms"],
+           "agent_steps_per_s": v * ww["n"], "us_per_launch": r["us_per_launch"], "timed_region_ms": r["ms_total"],
+           "check_replays_ms_min_max": r["check_replays_ms"],
            "roofline": {"achieved": gbs, "peak": peak, "frac": gbs / peak, "unit": "GB/s", "algorithmic_bytes_per_env_step": pu,
                         "env_steps_per_launch": r["envs_per_launch"], "map_cells_touched_per_env_step": tch, "traffic": load_traffic(name)}}
     if "e2e_s_per_step" in r:
@@ -859,7 +883,13 @@ def main():
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-extra", action="store_true", help="skip the supplementary workloads / CPU baseline")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy "
+                                                         "(rank 0's envs; float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -882,7 +912,8 @@ def main():
     sampler = ClockSampler(device.index)
     if rank == 0:
         sampler.start()
-    res = run_gpu_workload(cs, torch, args.workload, args.steps, args.warmup, device, rank, world)
+    res = run_gpu_workload(cs, torch, args.workload, args.steps, args.warmup, device, rank, world,
+                           dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
 
     ms_max = dist.max_over_ranks(res["ms_total"], device=device)
@@ -903,7 +934,7 @@ def main():
             try:
                 k = min(args.steps, 60 if name != "c5" else 20)
                 # (no host-buffer leg for c5 at its full size: 131072 envs x 80 KB of observations / state planes per step)
-                r = run_gpu_workload(cs, torch, name, k, 5, device, rank, world, want_e2e=(world == 1 and name != "c5"), burn_in_s=0.1)
+                r = run_gpu_workload(cs, torch, name, k, 5, device, rank, world, want_e2e=(world == 1 and name != "c5"), burn_in_steps=2000)
                 r["ms_per_step"] = dist.max_over_ranks(r["ms_per_step"], device=device)
                 r["us_per_launch"] = dist.max_over_ranks(r["us_per_launch"], device=device)
                 st = dist.allreduce_stats(r["stats"])
@@ -942,8 +973,8 @@ def main():
         "ms_per_step": ms_max / args.steps, "higher_is_better": True, "scaling": w.get("scaling", "weak"), "vs_baseline": None,
         "dtype": "f64", "data": "synthetic",
         "config": cfg,
-        "timed": {"replays_of_the_K_step_graph": res["timed_reps"], "region_ms": res["timed_region_ms"], "median_replay_ms": res["ms_total"],
-                  "min_replay_ms": res["ms_min"], "max_replay_ms": res["ms_max"], "lanes_per_env": res["lanes_per_env"], "streams": res["streams"]},
+        "timed": {"steps": args.steps, "region_ms": res["ms_total"], "burn_in_steps": res["burn_in_steps"],
+                  "check_replays_ms_min_max": res["check_replays_ms"], "lanes_per_env": res["lanes_per_env"], "streams": res["streams"]},
         "agent_steps_per_s": value * w["n"],
         "e2e": {"value": e2e_value, "unit": "env-steps/s", "h2d_bytes_per_step": res["h2d_bytes_per_step"],
                 "d2h_bytes_per_step": res["d2h_bytes_per_step"], "agent_steps_per_s": e2e_value * w["n"],
@@ -956,7 +987,7 @@ def main():
                      "kernel": kernel_name(w, res["lanes_per_env"], res["grouped"]),
                      "algorithmic_bytes_per_env_step": per_unit, "env_steps_per_launch": res["envs_per_launch"],
                      "us_per_launch": 1e6 * sec_per_launch, "map_cells_touched_per_env_step": touched,
-                     "note": "duration = median K-step replay / launches; launches of independent batches overlap when streams > 1"},
+                     "note": "duration = timed K-step replay / launches; launches of independent batches overlap when streams > 1"},
         "clocks": clocks,
         "episode_stats_allreduced": dict(zip(cs._lib.STAT_NAMES, [float(x) for x in stats.tolist()])),
         "stats_allreduce_us": allreduce_us,
@@ -967,7 +998,7 @@ def main():
                 if name == args.workload:
                     continue
                 try:
-                    r = run_gpu_workload(cs, torch, name, min(args.steps, 60), 5, device, 0, 1, want_e2e=True, burn_in_s=0.1)
+                    r = run_gpu_workload(cs, torch, name, min(args.steps, 60), 5, device, 0, 1, want_e2e=True, burn_in_steps=2000)
                     extra[name] = extra_entry(cs, torch, name, r, peak, device)
                 except Exception as exc:
                     extra[name] = {"error": repr(exc)}

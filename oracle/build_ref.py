@@ -1,10 +1,10 @@
 """Stages the UNMODIFIED reference into oracle/_ref/ -- TEST / BASELINE INFRASTRUCTURE.
 
 The reference (WZN1ng/Cooperative-Search) is pure Python: there is nothing to compile.  So that the CPU baseline of
-bench.py (`--impl reference`, `cpu_baseline`) can time the reference's own code path on the GPU box -- where
-/root/reference does not exist -- `__graft_entry__.build()` copies the files that path needs, byte for byte, from
-/root/reference into the git-ignored oracle/_ref/ (which travels to the box like the built .so files).  Nothing is
-edited; MANIFEST.json records the sha256 of every staged file.  Only tests/, smoke() and bench.py's CPU legs use it.
+bench.py (`--impl reference`, `cpu_baseline`) can time the reference's own code path on a machine the reference
+checkout is not on, `__graft_entry__.build()` copies the files that path needs, byte for byte, from the reference
+checkout (`source()`) into the git-ignored oracle/_ref/ (which a copy of the tree carries along).  Nothing is edited;
+MANIFEST.json records the sha256 of every staged file.  Only tests/, smoke() and bench.py's CPU legs use it.
 """
 import hashlib
 import json
@@ -12,7 +12,6 @@ import os
 import shutil
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = os.environ.get("COOPSEARCH_REFERENCE", "/root/reference")
 REF_DST = os.path.join(HERE, "_ref")
 # the env-step path and its caller (common/rollout.py + the Agents facade it needs for alg=random)
 FILES = [
@@ -25,17 +24,29 @@ FILES = [
 ]
 
 
+def source():
+    """The reference checkout: the COOPSEARCH_REFERENCE environment variable, else the reference_path that BASELINE.json
+    declares.  None when neither holds the reference."""
+    root = os.environ.get("COOPSEARCH_REFERENCE")
+    if not root:
+        with open(os.path.join(HERE, "..", "BASELINE.json")) as fh:
+            root = json.load(fh).get("reference_path")
+    return root if root and os.path.isfile(os.path.join(root, "env", "flight_env_easy.py")) else None
+
+
 def available():
     return os.path.isfile(os.path.join(REF_DST, "env", "flight_env_easy.py"))
 
 
 def stage(force=False):
-    """Copies the reference files into oracle/_ref/ when /root/reference is present.  Returns the staged root or None."""
-    if not os.path.isfile(os.path.join(REF_SRC, "env", "flight_env_easy.py")):
+    """Copies the reference files into oracle/_ref/ when the reference checkout is present.  Returns the staged root or
+    None."""
+    src_root = source()
+    if src_root is None:
         return REF_DST if available() else None
     manifest = {}
     for rel in FILES:
-        src, dst = os.path.join(REF_SRC, rel), os.path.join(REF_DST, rel)
+        src, dst = os.path.join(src_root, rel), os.path.join(REF_DST, rel)
         if not os.path.isfile(src):
             continue
         os.makedirs(os.path.dirname(dst), exist_ok=True)

@@ -1,8 +1,8 @@
 """Harness around the UNMODIFIED reference envs -- TEST INFRASTRUCTURE.
 
-Usable where ``/root/reference`` exists (the build container) or where the
-unmodified copies staged by ``oracle/build_ref.py`` under ``oracle/_ref`` exist
-(git-ignored; they travel to the GPU box like the built .so files).  It is used
+Usable where the reference checkout is present (``COOPSEARCH_REFERENCE``, else
+BASELINE.json's ``reference_path``: ``oracle/build_ref.py: source``), or where the
+unmodified copies staged from it under ``oracle/_ref`` exist (git-ignored).  It is used
 by ``tests/golden/make_golden.py`` to generate the committed golden fixtures, by
 the ``needs_reference`` CPU tests to pin the oracle restatement against the real
 thing, and by ``bench.py``'s CPU legs (the reference arm).  Nothing in the product
@@ -12,7 +12,7 @@ What it does:
   * injects stub ``matplotlib`` modules (the reference imports matplotlib at
     module top level: env/flight_env_easy.py:2-3, env/flight_env.py:2-3,
     env/search_env.py:4-5,49-53; matplotlib is not installed here);
-  * imports the reference env classes from ``/root/reference``;
+  * imports the reference env classes from that tree;
   * replaces the detection draw ``np.random.rand()`` (env/flight_env_easy.py:238,
     env/flight_env.py:248) by the keyed Philox draw of oracle/philox.py, reading
     the loop indices ``i`` (agent) and ``j`` (target) from the caller's frame.
@@ -25,19 +25,12 @@ import types
 
 import numpy as np
 
-from . import philox
+from . import build_ref, philox
 
 _STAGED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")     # oracle/build_ref.py: unmodified copies
 
 
-def _pick_root():
-    for root in (os.environ.get("COOPSEARCH_REFERENCE", "/root/reference"), _STAGED):
-        if os.path.isfile(os.path.join(root, "env", "flight_env_easy.py")):
-            return root
-    return "/root/reference"
-
-
-REFERENCE_ROOT = _pick_root()
+REFERENCE_ROOT = build_ref.source() or _STAGED
 
 
 def reference_available():

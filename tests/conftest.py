@@ -11,7 +11,7 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box via gpurun)")
-    config.addinivalue_line("markers", "needs_reference: needs the read-only reference tree (build container only)")
+    config.addinivalue_line("markers", "needs_reference: needs the reference checkout (COOPSEARCH_REFERENCE, else BASELINE.json reference_path)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -24,7 +24,7 @@ def pytest_collection_modifyitems(config, items):
         have_gpu = False
     for item in items:
         if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="reference tree not present on this box"))
+            item.add_marker(pytest.mark.skip(reason="no reference checkout (COOPSEARCH_REFERENCE, BASELINE.json reference_path) and no staged oracle/_ref"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
 

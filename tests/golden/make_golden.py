@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Generates tests/golden/*.npz by running the UNMODIFIED reference envs.
 
-Run in the build container only (needs /root/reference):
+Needs the reference checkout (COOPSEARCH_REFERENCE, else BASELINE.json's reference_path):
 
     python tests/golden/make_golden.py
 

@@ -26,7 +26,7 @@ def test_library_exports_every_symbol_of_the_header():
     assert lib.cs_launch_count() == 0          # nothing launched by loading
 
 
-def test_struct_sizes_match_the_header():
+def test_struct_sizes_match_the_header(tmp_path):
     """A C translation unit including the header reports the struct sizes the ctypes mirrors must have."""
     from coopsearch_b200 import _lib
     src = r'''
@@ -37,10 +37,9 @@ def test_struct_sizes_match_the_header():
         sizeof(cs_episode_buffers), sizeof(cs_policy_cfg), sizeof(cs_policy_weights), sizeof(cs_policy_io),
         sizeof(cs_spread_cfg), sizeof(cs_spread_buffers), sizeof(cs_flight_host_views)); return 0; }
     '''
-    exe = "/tmp/cs_sizes_%d" % os.getpid()
+    exe = str(tmp_path / "cs_sizes")
     subprocess.run(["gcc", "-x", "c", "-I", os.path.join(ROOT, "include"), "-o", exe, "-"], input=src.encode(), check=True)
     got = [int(v) for v in subprocess.run([exe], capture_output=True, check=True).stdout.split()]
-    os.remove(exe)
     want = [C.sizeof(t) for t in (_lib.FlightCfg, _lib.FlightBuffers, _lib.FlightHostIO, _lib.SearchCfg,
                                   _lib.SearchBuffers, _lib.SearchHostIO, _lib.EpisodeBuffers, _lib.PolicyCfg,
                                   _lib.PolicyWeights, _lib.PolicyIO, _lib.SpreadCfg, _lib.SpreadBuffers, _lib.FlightHostViews)]

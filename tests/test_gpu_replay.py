@@ -1,5 +1,5 @@
 """Device replay ring and replay statistics (SURVEY.md section 8f ranks 2 and 4) against the reference's own
-common/replay_buffer.py (imported from oracle/_ref or /root/reference) and its shipped result curves."""
+common/replay_buffer.py (imported from the reference checkout or oracle/_ref) and its shipped result curves."""
 import types
 
 import numpy as np

@@ -1,4 +1,4 @@
-"""Wide anchor of the C oracle on the UNMODIFIED reference (needs /root/reference or the staged oracle/_ref; skipped
+"""Wide anchor of the C oracle on the UNMODIFIED reference (needs the reference checkout or the staged oracle/_ref; skipped
 elsewhere): hundreds of fresh trajectories per env type, generated here by tests/golden/make_golden.py's own harness
 (MT19937 target layouts of the reference's reset injected, detection draws keyed), against the C oracle that the GPU
 parity tests at configuration size are checked with.  Everything is compared with np.array_equal -- float64 positions
