@@ -342,7 +342,7 @@ struct cs_policy {
     float* d_conv_w;
     size_t w_floats;
     float* d_w;
-    unsigned char* d_wtc;        // tensor-core weights (null where the tensor-core kernel does not apply: in_dim > 16)
+    unsigned char* d_wtc;        // tensor-core weights (packed for every allowed input width, <= kTcK1 = 32)
 };
 
 extern "C" {

@@ -2,10 +2,12 @@
 action choice of Agents.choose_action (agent/agent.py:33-97) for every (env, agent) row of a vectorised env at once,
 in one kernel launch (csrc/policy.cu, csrc/policy_tc.cuh).  The reference evaluates one (1, in) row per agent per step.
 
-precision "bf16" (default where the input width is <= 16): the five GEMMs of a 128-row tile run on the tcgen05 tensor
-cores with bf16 operands, fp32 accumulators in tensor memory and an fp32 hidden state; "fp32": the CUDA-core kernel
-that equals the reference's torch modules to 1e-5.  alg: "q" = masked argmax / epsilon-greedy (qmix, vdn; dop's actor is
-the same network class with the actor's weights), "reinforce" = softmax sampling (agent/agent.py:77-97)."""
+precision "bf16" (the default, for every allowed input width up to 32): the five GEMMs of a 128-row tile run on the
+tcgen05 tensor cores with bf16 operands, fp32 accumulators in tensor memory and an fp32 hidden state; "fp32": the
+CUDA-core kernel that equals the reference's torch modules to 1e-5.  Both are held to a float64 reference with
+per-element error bounds (oracle/policy_ref.py, tests/test_gpu_policy_reference.py).
+alg: "q" = masked argmax / epsilon-greedy (qmix, vdn; dop's actor is the same network class with the actor's weights),
+"reinforce" = softmax sampling (agent/agent.py:77-97)."""
 import ctypes as C
 
 import numpy as np
