@@ -256,17 +256,21 @@ __device__ __forceinline__ float rcp_approx(float x) {
 }
 
 // One cell of the belief update (flight_env.py:291-292), p' = percent*(1-d)*p / ((1-d)*p + (1-p)), fp32 and branch
-// free: c = corners-in-view * (1-d)/4 (0 for an untouched cell), u = 1 for an untouched cell else 0, so that
-// r = (c*p) * rcp(den) + u*p is the update for a touched cell and p itself for an untouched one.  The reference's own
+// free: w = corners-in-view / 4 (exact; 0 for an untouched cell), u = 1 for an untouched cell else 0, so that
+// r = (w*qp) * rcp(den) + u*p is the update for a touched cell and p itself for an untouched one.  q = 1-d enters as
+// the pair qf + ql (qf = fl32(q), ql = fl32(q - qf)), so that qp is q*p to fp32 accuracy: q rounded to fp32 alone
+// would shift every update by |fl32(q) - q| / q in the same direction (1.5e-8 at d = 0.9, 1.3e-8 at d = 0.05), and
+// a cell collects that once per call for as long as it stays in view (DESIGN section 4.4).  The reference's own
 // grouping (1-d)*p + (1-p) matters: 1-p is exact near p = 1.  A cell at exactly 1 (a found target) must map to
 // exactly percent -- in particular stay exactly 1 while all four corners are in view -- because the map's derivative
-// there is 10 and any seed error would grow tenfold per step; the callers take that case exactly
+// there is 1/q and any seed error would grow by that factor per step; the callers take that case exactly
 // (values never approach 1 from below: p' <= p).  The fused kernel evaluates the same operations two cells at a time
 // (FMUL2 / FADD2 / FFMA2), bit for bit the same results.
-__device__ __forceinline__ float belief_cell(float pv, float c, float u, float qf) {
-    const float num = c * pv;                                   // percent*(1-d)*p            (:292)
+__device__ __forceinline__ float belief_cell(float pv, float w, float u, float qf, float ql) {
+    const float qp = fmaf(qf, pv, ql * pv);                     // (1-d)*p
+    const float num = w * qp;                                   // percent*(1-d)*p
     const float keep = u * pv;
-    const float den = fmaf(qf, pv, 1.0f - pv);                  // (1-d)*p + (1-p)
+    const float den = qp + (1.0f - pv);                         // (1-d)*p + (1-p)
     return fmaf(num, rcp_approx(den), keep);
 }
 

@@ -138,14 +138,13 @@ void host_heading_sincos(const HeadingLut& lut, double h, double* sn, double* c,
 
 // Table of the fused belief-map sweep (flight_map.cuh): the 10 corner bits of a float4 of cells -- x0 = corners
 // j..j+4 of corner row i (bits 0..4), x1 = the same of corner row i+1 (bits 5..9) -- give, for each of the 4 cells,
-// c = corners-in-view * (1-d)/4 and u = (corners-in-view == 0).  fp32 products exactly as the device would form them.
-void build_cell_lut(float qf, std::vector<float>* out) {
-    const float kq = 0.25f * qf;
+// w = corners-in-view / 4 (exact) and u = (corners-in-view == 0).  (1-d) is applied by the sweep as an fp32 pair.
+void build_cell_lut(std::vector<float>* out) {
     out->assign(1024 * 8, 0.0f);
     for (unsigned idx = 0; idx < 1024; ++idx)
         for (int k = 0; k < 4; ++k) {
             const int cnt = __builtin_popcount(idx & (0x63u << k));
-            (*out)[idx * 8 + k] = (float)cnt * kq;
+            (*out)[idx * 8 + k] = 0.25f * (float)cnt;
             (*out)[idx * 8 + 4 + k] = cnt == 0 ? 1.0f : 0.0f;
         }
 }
@@ -220,7 +219,7 @@ int flight_alloc(cs_flight* h) {
             }
         }
         std::vector<float> cells;
-        build_cell_lut((float)p.q_miss, &cells);
+        build_cell_lut(&cells);
         CS_CUDA(cudaMalloc(&h->d_lut_cells, cells.size() * sizeof(float)));
         CS_CUDA(cudaMemcpy(h->d_lut_cells, cells.data(), cells.size() * sizeof(float), cudaMemcpyHostToDevice));
         p.lut_cells = h->d_lut_cells;

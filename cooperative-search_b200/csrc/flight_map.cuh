@@ -14,7 +14,7 @@
 //      row ORs its five corner rows and lists the touched tiles of that row (prefix sum over the env's lanes).
 //  (3) sweep: the env's lanes walk the tile list, four lanes per tile, one float4 (4 cells of one map row) per lane
 //      and four tiles in flight per lane; the 10 corner bits of a float4 index a 1024-entry table (32 KB, L1
-//      resident) that yields the four weights corners*(1-d)/4 and the four "untouched" flags, and the update runs as
+//      resident) that yields the four weights corners/4 and the four "untouched" flags, and the update runs as
 //      packed fp32 pairs (FMUL2 / FADD2 / FFMA2 + MUFU.RCP).  Untouched float4s are neither read nor written.
 //  (4) the cells of targets found by THIS call become 1 where percent > 0 (:288-289), after the sweep.
 // The fused form runs inside the thread-per-env step kernel (flight_tpe.cu): the env's 8 lanes just computed the
@@ -42,6 +42,12 @@ __device__ __forceinline__ float2 f2_sub(float2 a, float2 b) {
         : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
     return d;
 }
+__device__ __forceinline__ float2 f2_add(float2 a, float2 b) {
+    float2 d;
+    asm("{\n\t.reg .b64 ra, rb, rd;\n\tmov.b64 ra, {%2, %3};\n\tmov.b64 rb, {%4, %5};\n\tadd.rn.f32x2 rd, ra, rb;\n\tmov.b64 {%0, %1}, rd;\n\t}"
+        : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
+    return d;
+}
 __device__ __forceinline__ float2 f2_fma(float2 a, float2 b, float2 c) {
     float2 d;
     asm("{\n\t.reg .b64 ra, rb, rc, rd;\n\tmov.b64 ra, {%2, %3};\n\tmov.b64 rb, {%4, %5};\n\tmov.b64 rc, {%6, %7};\n\tfma.rn.f32x2 rd, ra, rb, rc;\n\tmov.b64 {%0, %1}, rd;\n\t}"
@@ -55,9 +61,10 @@ __device__ __forceinline__ float f_max3(float a, float b, float c) {
 }
 
 // two cells of belief_cell() at once
-__device__ __forceinline__ float2 belief_pair(float2 pv, float2 c, float2 u, float qf) {
-    const float2 num = f2_mul(c, pv), keep = f2_mul(u, pv);
-    const float2 den = f2_fma(make_float2(qf, qf), pv, f2_sub(make_float2(1.0f, 1.0f), pv));
+__device__ __forceinline__ float2 belief_pair(float2 pv, float2 w, float2 u, float qf, float ql) {
+    const float2 qp = f2_fma(make_float2(qf, qf), pv, f2_mul(make_float2(ql, ql), pv));
+    const float2 num = f2_mul(w, qp), keep = f2_mul(u, pv);
+    const float2 den = f2_add(qp, f2_sub(make_float2(1.0f, 1.0f), pv));
     return f2_fma(num, make_float2(rcp_approx(den.x), rcp_approx(den.y)), keep);
 }
 
@@ -66,10 +73,10 @@ __device__ __forceinline__ int f4_corners(unsigned idx, int k) { return __popc(i
 
 // One float4 of cells: old values v, corner bits idx (!= 0).  Exact cases: a cell at exactly 1 -> exactly percent; with
 // detect_prob = 1 (qf = 0: 0/0 = nan, like the reference) the untouched cells of the float4 keep their bits.
-__device__ __forceinline__ float4 belief_f4(const FlightParams& p, float4 v, unsigned idx, float qf) {
+__device__ __forceinline__ float4 belief_f4(const FlightParams& p, float4 v, unsigned idx, float qf, float ql) {
     const float4 c = __ldg(p.lut_cells + 2 * idx), u = __ldg(p.lut_cells + 2 * idx + 1);
-    const float2 lo = belief_pair(make_float2(v.x, v.y), make_float2(c.x, c.y), make_float2(u.x, u.y), qf);
-    const float2 hi = belief_pair(make_float2(v.z, v.w), make_float2(c.z, c.w), make_float2(u.z, u.w), qf);
+    const float2 lo = belief_pair(make_float2(v.x, v.y), make_float2(c.x, c.y), make_float2(u.x, u.y), qf, ql);
+    const float2 hi = belief_pair(make_float2(v.z, v.w), make_float2(c.z, c.w), make_float2(u.z, u.w), qf, ql);
     float4 r = make_float4(lo.x, lo.y, hi.x, hi.y);
     if (qf == 0.0f) {
         r.x = (u.x != 0.0f) ? v.x : r.x; r.y = (u.y != 0.0f) ? v.y : r.y;
@@ -137,7 +144,7 @@ __device__ __forceinline__ void fused_map_phase(const FlightParams& p, int e, in
     unsigned short* list = reinterpret_cast<unsigned short*>(S + p.fm_list);
     int* clo = reinterpret_cast<int*>(S + p.fm_clo);
     float* map = p.prob_map + (size_t)e * p.map_stride;
-    const float qf = (float)p.q_miss;
+    const float qf = (float)p.q_miss, ql = (float)(p.q_miss - (double)qf);      // q = 1-d as an fp32 pair
     const unsigned long long cellmask = (1ull << M) - 1ull;          // M <= 63
     const int r4 = kk & 3, quad = kk >> 2;
     unsigned touched = 0;
@@ -212,7 +219,7 @@ __device__ __forceinline__ void fused_map_phase(const FlightParams& p, int e, in
                 }
 #pragma unroll
                 for (int u = 0; u < U; ++u)
-                    if (idx[u]) __stcg(reinterpret_cast<float4*>(map + off[u]), belief_f4(p, v[u], idx[u], qf));
+                    if (idx[u]) __stcg(reinterpret_cast<float4*>(map + off[u]), belief_f4(p, v[u], idx[u], qf, ql));
             }
         }
         __syncwarp();                                                // sweep stores before the stores below (same cells)
@@ -334,7 +341,7 @@ static __global__ void __launch_bounds__(kMapThreads) flight_map_generic_kernel(
     double* xy = reinterpret_cast<double*>(S + p.ms_xy);
     int* hit = reinterpret_cast<int*>(S + p.ms_hit);
     float* map = p.prob_map + (size_t)e * p.map_stride;
-    const float qf = (float)p.q_miss, kq = 0.25f * qf;
+    const float qf = (float)p.q_miss, ql = (float)(p.q_miss - (double)qf);
     const int colk = lane & 15, half = lane >> 4;
     unsigned touched = 0;
     for (int job = (m1.w & 1u) ? 0 : 1; job < 2; ++job) {
@@ -377,7 +384,7 @@ static __global__ void __launch_bounds__(kMapThreads) flight_map_generic_kernel(
                     const int cnt = __popc(bits);
                     float* cellp = map + tile_off(p.tiles, i, j);
                     const float pv = *cellp;
-                    float v = belief_cell(pv, (float)cnt * kq, 0.0f, qf);
+                    float v = belief_cell(pv, 0.25f * (float)cnt, 0.0f, qf, ql);
                     if (pv == 1.0f && qf != 0.0f) v = 0.25f * (float)cnt;    // see belief_cell: the exact case
                     for (int k = 0; k < nh; ++k)
                         if (hit[k] == i * M + j) v = 1.0f;                    // found by THIS call (:288-289)
