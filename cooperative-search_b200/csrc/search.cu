@@ -45,6 +45,8 @@ struct SearchParams {
     uint8_t* terminated;
     int32_t* target_find;
     double* stats;
+    double* ep_reward;               // [E] fp64 sum of the running episode's step rewards -> CS_STAT_EP_REWARD
+    int place_batches;               // cap on 128-candidate batches of target placement (search_init)
 };
 
 struct SearchSmem {
@@ -80,6 +82,11 @@ size_t smem_base_bytes(const SearchParams& p) {
     const size_t used = sizeof(uint32_t) * (size_t)(3 * p.M * p.W) + sizeof(int32_t) * (size_t)(2 * p.n + 2 * kThreads + 8 + p.S + 2 * p.R + 1);
     return (used + 15) & ~(size_t)15;
 }
+// cells of the target_mode 1 edge band: x or y <= M/4 or >= 3M/4 (search_env.py:96-104)
+int search_band_cells(int M) {
+    const int inner = 3 * M / 4 - M / 4 - 1;
+    return M * M - (inner > 0 ? inner * inner : 0);
+}
 // v / d with magic = ceil(2^32 / d); d == 1 gives magic 2^32 -> stored as 0 -> identity
 __device__ __forceinline__ int fastdiv(int v, uint32_t magic) { return magic ? (int)__umulhi((uint32_t)v, magic) : v; }
 
@@ -105,9 +112,10 @@ __device__ void search_reset(const SearchParams& p, const SearchSmem& s, int e, 
         // Rejection sampling in candidate order k = 0,1,...: candidate k is Philox(env, episode, k) ->
         // (w0 % M, w1 % M); accepted when the cell is free (mode 1: and in the edge band) -- the accept rule of
         // search_env.py:86-104.  Philox for a batch of candidates in parallel, acceptance in order by thread 0.
+        // cs_search_create refuses requests that cannot be met; place_batches bounds the loop so that a met request
+        // always completes (search_init states the bound) and nothing can spin forever
         const int lo = M / 4, hi = 3 * M / 4;
-        // the reference loops forever when the request cannot be satisfied; bound it (a hung GPU helps nobody)
-        for (int batch = 0; batch < (1 << 14); ++batch) {
+        for (int batch = 0; batch < p.place_batches; ++batch) {
             const int base = s.scal[SC_NEXTK];
             const cs_u4 w = cs_philox4x32_10(env_id, ((uint32_t)episode & 0xFFFFu) << 16, (uint32_t)(base + tid), 0u, p.seed,
                                              cs_stream_key(CS_STREAM_SEARCH, (uint32_t)episode));
@@ -152,6 +160,7 @@ __device__ void search_reset(const SearchParams& p, const SearchSmem& s, int e, 
     }
     if (tid == 0) {
         cnt_local[CNT_FIND] = 0; cnt_local[CNT_TIME] = 0; cnt_local[CNT_FLAGS] = 0; cnt_local[CNT_EPISODE] = episode;
+        p.ep_reward[e] = 0.0;
     }
     __syncthreads();
 }
@@ -263,6 +272,7 @@ __global__ void __launch_bounds__(kThreads) search_kernel(const SearchParams p, 
     extern __shared__ __align__(16) unsigned char raw[];
     __shared__ int32_t cnt[4];
     __shared__ double s_red[kThreads / 32];
+    __shared__ double s_ep_reward;
     const SearchSmem s = carve(p, raw);
     const int tid = threadIdx.x, e = blockIdx.x, M = p.M, W = p.W, n = p.n;
     const int rows = M * W;
@@ -299,7 +309,6 @@ __global__ void __launch_bounds__(kThreads) search_kernel(const SearchParams p, 
     bool emit = false, bits_dirty = false;
     if (MODE == MODE_STEP) {
         bool done = (cnt[CNT_FLAGS] & SF_DONE) != 0;
-        float rew_out = 0.f;
         if (!done) {
             int32_t* fq = p.freq + (size_t)e * M * M;
             const int t1 = cnt[CNT_TIME] + 1;
@@ -334,6 +343,7 @@ __global__ void __launch_bounds__(kThreads) search_kernel(const SearchParams p, 
                 }
             }
             __syncthreads();
+            if (tid == 32) s_ep_reward = p.ep_reward[e];     // the episode's reward so far, loaded while detection runs
             // ---- reward: sum_i 1/freq[p_i] in fp64 (:257-259)
             double part = 0.0;
             for (int a = tid; a < n; a += kThreads) part += 1.0 / (double)__ldcg(&fq[s.pos[2 * a] * M + s.pos[2 * a + 1]]);
@@ -359,26 +369,29 @@ __global__ void __launch_bounds__(kThreads) search_kernel(const SearchParams p, 
             }
             __syncthreads();
             const int newf = s.scal[SC_NEWFOUND];
-            double fsum = 0.0;
-            for (int k = 0; k < kThreads / 32; ++k) fsum += s_red[k];
             const int found = cnt[CNT_FIND] + newf;
             const bool term = found >= p.m;                                  // (:270-271)
-            rew_out = (float)(-1.0 + fsum + 10.0 * (double)newf);            // MOVE_COST + freq + REWARD_FIND (:250-265)
             __syncthreads();
             if (tid == 0) {
+                double fsum = 0.0;
+                for (int k = 0; k < kThreads / 32; ++k) fsum += s_red[k];
+                const double rew = -1.0 + fsum + 10.0 * (double)newf;       // MOVE_COST + freq + REWARD_FIND (:250-265)
                 cnt[CNT_FIND] = found;
                 cnt[CNT_TIME] = t1;
                 cnt[CNT_FLAGS] |= (term ? SF_DONE : 0) | (s.scal[SC_ILLEGAL] ? SF_ILLEGAL : 0);
                 // no per-step statistic: a same-address atomic per CTA per step serialises in L2; env_steps is
                 // assembled by cs_search_stats from finished-episode lengths + live time_steps
                 if (s.scal[SC_ILLEGAL]) atomicAdd(p.stats + CS_STAT_ILLEGAL, 1.0);
+                const double ep_rew = s_ep_reward + rew;                     // fp64, before the fp32 cast of the output
+                p.ep_reward[e] = ep_rew;
                 if (term) {
                     atomicAdd(p.stats + CS_STAT_EPISODES, 1.0);
+                    atomicAdd(p.stats + CS_STAT_EP_REWARD, ep_rew);
                     atomicAdd(p.stats + CS_STAT_TARGETS_FOUND, (double)found);
                     atomicAdd(p.stats + CS_STAT_WINS, 1.0);
                     atomicAdd(p.stats + CS_STAT_EP_LEN, (double)t1);
                 }
-                p.reward[e] = rew_out;
+                p.reward[e] = (float)rew;
                 p.terminated[e] = term ? 1 : 0;
                 p.target_find[e] = found;
             }
@@ -468,6 +481,9 @@ int cs_search_create(const cs_search_cfg* cfg, cs_search** out) {
     CS_REQUIRE(cfg->agent_mode >= 0 && cfg->agent_mode <= 2, "Unknown agent mode");          // search_env.py:180
     CS_REQUIRE(cfg->target_mode == 0 || cfg->target_mode == 1, "Unknown target mode");        // :143 (modes 2,3: inject cells)
     CS_REQUIRE(cfg->agent_mode != 2 || cfg->n_agents >= 2, "agent_mode 2 divides by n_agents-1 (search_env.py:171)");
+    CS_REQUIRE(cfg->target_mode != 1 || cfg->target_num <= search_band_cells(cfg->map_size),
+               "target_mode 1: target_num %d exceeds the %d cells of the edge band (the reference never finishes placing them)",
+               cfg->target_num, search_band_cells(cfg->map_size));
     {
         const int L = (int)ceil(sqrt((double)cfg->n_agents));
         CS_REQUIRE(cfg->agent_mode == 2 || L <= cfg->map_size, "agents do not fit the map");
@@ -514,6 +530,16 @@ int search_init(cs_search* h) {
             cur_limit = h->smem_bytes;
         }
     }
+    {
+        // Target placement draws uniform candidates over all M^2 cells and accepts the eligible free ones (all cells; mode 1:
+        // the edge band).  A given eligible cell is missed by N candidates with probability (1 - 1/M^2)^N <= e^(-N/M^2);
+        // over the Q eligible cells, N = M^2 (ln Q + c) leaves one unvisited with probability <= e^-c (the coupon-collector
+        // tail).  Every eligible cell visited means every accepted request (m <= Q) is placed in full; c = 70 puts a
+        // shortfall at <= 4e-31 per reset.  Envs stop at the m-th accepted cell (c5, m = 1000 of 4096: ~1150 candidates).
+        const double MM = (double)p.M * p.M;
+        const double Q = p.target_mode == 1 ? (double)search_band_cells(p.M) : MM;
+        p.place_batches = (int)ceil(MM * (log(Q) + 70.0) / kThreads);
+    }
     const size_t E = (size_t)p.E, rows = (size_t)p.M * p.W, MM = (size_t)p.M * p.M;
 #define CS_ALLOC0(ptr, bytes)                                   \
     CS_CUDA(cudaMalloc(reinterpret_cast<void**>(&(ptr)), (bytes))); \
@@ -532,6 +558,7 @@ int search_init(cs_search* h) {
     CS_ALLOC0(p.stats, CS_NUM_STATS * sizeof(double));
     CS_ALLOC0(h->d_actions, E * p.n);
     CS_ALLOC0(h->d_live, sizeof(double));
+    CS_ALLOC0(p.ep_reward, E * sizeof(double));
 #undef CS_ALLOC0
     // episode counter starts at -1 so that the first reset opens episode 0
     CS_CUDA(cudaMemset2D(p.counters + CNT_EPISODE, 4 * sizeof(int32_t), 0xFF, sizeof(int32_t), E));
@@ -547,7 +574,7 @@ void cs_search_destroy(cs_search* h) {
     SearchParams& p = h->p;
     cudaFree(p.pos); cudaFree(p.target_bits); cudaFree(p.unfound_bits); cudaFree(p.freq); cudaFree(p.counters);
     cudaFree(p.obs); cudaFree(p.state); cudaFree(p.avail); cudaFree(p.reward); cudaFree(p.terminated);
-    cudaFree(p.target_find); cudaFree(p.stats); cudaFree(h->d_cells); cudaFree(h->d_actions); cudaFree(h->d_live);
+    cudaFree(p.target_find); cudaFree(p.stats); cudaFree(p.ep_reward); cudaFree(h->d_cells); cudaFree(h->d_actions); cudaFree(h->d_live);
     delete h;
 }
 

@@ -109,7 +109,25 @@ class VecSearchEnv:
                     cells.append([x, y])
         if len(cells) != self.target_num:
             raise CoopSearchError("target file holds %d cells, target_num is %d" % (len(cells), self.target_num))
+        self._check_cells(np.array(cells, np.int64)[None], "target file %s" % filename)
         return np.broadcast_to(np.array(cells, np.int32), (self.num_envs, self.target_num, 2)).copy()
+
+    def _check_cells(self, cells, what):
+        """Target cells [E,m,2] must lie on the map and be distinct within an env: the reference counts found targets per
+        cell entry and would never reach target_num (search_env.py:263-271), while the bit rows hold one bit per cell."""
+        M = self.map_size
+        if cells.ndim != 3 or cells.shape[2] != 2:
+            raise CoopSearchError("%s: cells must have shape (num_envs, target_num, 2)" % what)
+        off = (cells < 0).any(-1) | (cells >= M).any(-1)
+        if off.any():
+            e, k = [int(v) for v in np.argwhere(off)[0]]
+            raise CoopSearchError("%s: cell %s (env %d, target %d) lies off the %dx%d map"
+                                  % (what, tuple(int(v) for v in cells[e, k]), e, k, M, M))
+        key = np.sort(cells[..., 0] * M + cells[..., 1], axis=1)
+        dup = key[:, 1:] == key[:, :-1]
+        if dup.any():
+            e, k = [int(v) for v in np.argwhere(dup)[0]]
+            raise CoopSearchError("%s: env %d lists cell (%d, %d) more than once" % (what, e, key[e, k] // M, key[e, k] % M))
 
     def _cells_from_circles(self):
         """target_mode 2 (search_env.py:106-123): host-side sampling from the circle dictionary with a
@@ -141,6 +159,9 @@ class VecSearchEnv:
         """reset (search_env.py:69-183).  `init` is accepted for signature parity; the freq map is never
         cleared either way (:39 vs :70-80).  cells: optional [E,m,2] int target cells to inject."""
         flags = 0
+        if cells is not None:
+            self._check_cells((cells.detach().cpu().numpy() if torch.is_tensor(cells) else np.asarray(cells)).astype(np.int64),
+                              "reset(cells=...)")
         if cells is None and self.target_mode == 3:
             cells = self._fixed_cells
         if cells is None and self.target_mode == 2:

@@ -174,6 +174,11 @@ class FlightBatch:
 
 
 class SearchBatch:
+    """E env instances of the search_env oracle, stepped in C.  With auto_reset a terminating env is reset inside the
+    step call, as the kernel does.  After step(): reward / terminated / target_find / terms describe that call's step (of
+    the finished episode, where one ended); terms[e] = (-1, 1/freq of agents 0..n-1, 10 * targets found) are the reward's
+    summands, zero for an env that did not step.  Everything else holds the state after the call."""
+
     def __init__(self, spec, seed, env_id_base, num_envs, auto_reset=False):
         self.spec = spec
         self.E = E = int(num_envs)
@@ -190,6 +195,8 @@ class SearchBatch:
         self.counters[:, 3] = -1
         self.reward = np.zeros(E)
         self.terminated = np.zeros(E, np.uint8)
+        self.target_find = np.zeros(E, np.int32)
+        self.terms = np.zeros((E, n + 2))
 
     def reset(self, cells=None, mask=None):
         if cells is not None:
@@ -208,17 +215,29 @@ class SearchBatch:
         _fanout(self.E, lambda e0, e1: f(C.byref(self.cs), e1 - e0, self.base + e0, _p(sl(a, e0, e1)), _p(self.pos[e0:e1]),
                                          _p(self.cells[e0:e1]), _p(self.tmap[e0:e1]), _p(self.found[e0:e1]),
                                          _p(self.freq[e0:e1]), _p(self.counters[e0:e1]), _p(self.reward[e0:e1]),
-                                         _p(self.terminated[e0:e1])))
+                                         _p(self.terminated[e0:e1]), _p(self.terms[e0:e1]), _p(self.target_find[e0:e1])))
         return self.reward, self.terminated
 
-    def views(self, want_obs=True, want_state=True):
+    def views(self, want_obs=True, want_state=True, envs=None):
+        """(obs, state, avail) of every env, or of the envs listed in `envs` (in that order)."""
         s = self.spec
         n, M, S = s.n_agents, s.map_size, 2 * s.view_range - 1
-        obs = np.zeros((self.E, n, S * S + 2), np.float32) if want_obs else None
-        state = np.zeros((self.E, 2 * M * M), np.float32) if want_state else None
-        avail = np.zeros((self.E, n, 4), np.uint8)
+        rows = np.arange(self.E) if envs is None else np.asarray(envs, np.int64).reshape(-1)
+        pos = self.pos if envs is None else np.ascontiguousarray(self.pos[rows])
+        tmap = self.tmap if envs is None else np.ascontiguousarray(self.tmap[rows])
+        R = len(rows)
+        obs = np.zeros((R, n, S * S + 2), np.float32) if want_obs else None
+        state = np.zeros((R, 2 * M * M), np.float32) if want_state else None
+        avail = np.zeros((R, n, 4), np.uint8)
         f = lib().os_views
         sl = lambda arr, e0, e1: None if arr is None else arr[e0:e1]
-        _fanout(self.E, lambda e0, e1: f(C.byref(self.cs), e1 - e0, _p(self.pos[e0:e1]), _p(self.tmap[e0:e1]),
-                                         _p(sl(obs, e0, e1)), _p(sl(state, e0, e1)), _p(avail[e0:e1])))
+        _fanout(R, lambda e0, e1: f(C.byref(self.cs), e1 - e0, _p(pos[e0:e1]), _p(tmap[e0:e1]),
+                                    _p(sl(obs, e0, e1)), _p(sl(state, e0, e1)), _p(avail[e0:e1])))
         return obs, state, avail
+
+    def unfound_map(self):
+        """[E, M, M] u8: target cells not found yet (the kernel's unfound bit rows)."""
+        out = self.tmap.copy()
+        e, k = np.nonzero(self.found)
+        out[e, self.cells[e, k, 0], self.cells[e, k, 1]] = 0
+        return out

@@ -357,35 +357,51 @@ static void search_place_targets(const os_spec* s, uint32_t env_id, uint32_t epi
     }
 }
 
-void os_reset(const os_spec* s, int E, uint32_t base, const uint8_t* mask, int keep_targets, int32_t* pos, int32_t* cells,
-              uint8_t* tmap, uint8_t* found, int32_t* freq, int32_t* counters) {
+/* reset of env e (search_env.py:69-183, init=False): the next episode, its targets, agents at their start cells */
+static void search_reset_env(const os_spec* s, int e, uint32_t env_id, int keep_targets, int32_t* pos, int32_t* cells,
+                             uint8_t* tmap, uint8_t* found, int32_t* freq, int32_t* counters) {
     const int M = s->M;
-    for (int e = 0; e < E; ++e) {
-        if (mask && !mask[e]) continue;
-        int32_t* ct = counters + (size_t)e * 4;
-        uint8_t* tm = tmap + (size_t)e * M * M;
-        ct[0] = 0; ct[1] = 0; ct[2] = 0; ct[3] += 1;
-        memset(tm, 0, (size_t)M * M);
-        memset(found + (size_t)e * s->m, 0, s->m);
-        if (keep_targets) {
-            for (int k = 0; k < s->m; ++k) tm[cells[((size_t)e * s->m + k) * 2] * M + cells[((size_t)e * s->m + k) * 2 + 1]] = 1;
-        } else {
-            search_place_targets(s, base + e, (uint32_t)ct[3], cells + (size_t)e * s->m * 2, tm);
-        }
-        search_place_agents(s, pos + (size_t)e * s->n * 2, freq + (size_t)e * M * M);
+    int32_t* ct = counters + (size_t)e * 4;
+    uint8_t* tm = tmap + (size_t)e * M * M;
+    ct[0] = 0; ct[1] = 0; ct[2] = 0; ct[3] += 1;
+    memset(tm, 0, (size_t)M * M);
+    memset(found + (size_t)e * s->m, 0, s->m);
+    if (keep_targets) {
+        for (int k = 0; k < s->m; ++k) tm[cells[((size_t)e * s->m + k) * 2] * M + cells[((size_t)e * s->m + k) * 2 + 1]] = 1;
+    } else {
+        search_place_targets(s, env_id, (uint32_t)ct[3], cells + (size_t)e * s->m * 2, tm);
     }
+    search_place_agents(s, pos + (size_t)e * s->n * 2, freq + (size_t)e * M * M);
 }
 
+void os_reset(const os_spec* s, int E, uint32_t base, const uint8_t* mask, int keep_targets, int32_t* pos, int32_t* cells,
+              uint8_t* tmap, uint8_t* found, int32_t* freq, int32_t* counters) {
+    for (int e = 0; e < E; ++e)
+        if (!mask || mask[e]) search_reset_env(s, e, base + e, keep_targets, pos, cells, tmap, found, freq, counters);
+}
+
+/* step (search_env.py:246-296).  terms (may be NULL): [E][n+2] the reward's terms of this call, -1, 1/freq of each agent
+ * and 10 * (targets found), zeros for an env that did not step; find_out (may be NULL): [E] target_find after the step of
+ * the finished episode.  With s->auto_reset a terminating env is reset within the call, like the kernel: counters, agents,
+ * targets and found flags then hold the new episode, reward / terminated / terms / find_out the finished one's step. */
 void os_step(const os_spec* s, int E, uint32_t base, const uint8_t* actions, int32_t* pos, int32_t* cells, uint8_t* tmap,
-             uint8_t* found, int32_t* freq, int32_t* counters, double* reward, uint8_t* terminated) {
+             uint8_t* found, int32_t* freq, int32_t* counters, double* reward, uint8_t* terminated, double* terms,
+             int32_t* find_out) {
     const int n = s->n, m = s->m, M = s->M, R2 = s->R * s->R;
-    (void)tmap;
     for (int e = 0; e < E; ++e) {
         int32_t* ct = counters + (size_t)e * 4;
         int32_t* p = pos + (size_t)e * n * 2;
         int32_t* fq = freq + (size_t)e * M * M;
-        if (ct[2] & 1) { reward[e] = 0; terminated[e] = 1; continue; }
+        double* tr = terms ? terms + (size_t)e * (n + 2) : NULL;
+        if (tr) memset(tr, 0, sizeof(double) * (size_t)(n + 2));
+        if (ct[2] & 1) {
+            reward[e] = 0; terminated[e] = 1;
+            if (find_out) find_out[e] = ct[0];
+            if (s->auto_reset) search_reset_env(s, e, base + e, 0, pos, cells, tmap, found, freq, counters);
+            continue;
+        }
         double rew = -1;
+        int newfound = 0;
         ct[1] += 1;
         for (int i = 0; i < n; ++i) {
             uint8_t a;
@@ -413,19 +429,24 @@ void os_step(const os_spec* s, int E, uint32_t base, const uint8_t* actions, int
         for (int i = 0; i < n; ++i) {
             const int xa = p[2 * i], ya = p[2 * i + 1];
             rew += 1 / (double)fq[xa * M + ya];
+            if (tr) tr[1 + i] = 1 / (double)fq[xa * M + ya];
             for (int k = 0; k < m; ++k) {
                 const int dx = cells[((size_t)e * m + k) * 2] - xa, dy = cells[((size_t)e * m + k) * 2 + 1] - ya;
                 if (dx * dx + dy * dy <= R2 && !found[(size_t)e * m + k]) {
                     rew += 10;
                     found[(size_t)e * m + k] = 1;
                     ct[0] += 1;
+                    ++newfound;
                 }
             }
         }
+        if (tr) { tr[0] = -1; tr[n + 1] = 10.0 * newfound; }
         const int term = ct[0] >= m;
         if (term) ct[2] |= 1;
         reward[e] = rew;
         terminated[e] = (uint8_t)term;
+        if (find_out) find_out[e] = ct[0];
+        if (term && s->auto_reset) search_reset_env(s, e, base + e, 0, pos, cells, tmap, found, freq, counters);
     }
 }
 

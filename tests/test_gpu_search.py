@@ -64,7 +64,8 @@ def test_search_matches_reference_golden(name):
 
 @pytest.mark.parametrize("n,m,M,R,am,tm", [(3, 15, 50, 7, 0, 0), (64, 1000, 64, 7, 0, 0), (9, 40, 33, 5, 1, 1), (6, 25, 70, 4, 2, 0)])
 def test_search_matches_c_oracle(n, m, M, R, am, tm):
-    """Device-side target placement + random legal policy in-kernel vs the C oracle, with auto-reset."""
+    """Device-side target placement + random legal policy in-kernel vs the C oracle, without auto-reset (the benchmarked
+    auto-reset path, whole episodes and the statistics: test_gpu_search_reference.py)."""
     import coopsearch_b200 as cs
     E, T, seed, base = 40, 90, 13, 4000
     spec = SearchSpec(n_agents=n, target_num=m, map_size=M, view_range=R, agent_mode=am, target_mode=tm)
