@@ -21,6 +21,7 @@ namespace {
 constexpr int kH = 64;                 // args.rnn_hidden_dim (common/arguments.py)
 constexpr int kPolicyThreads = 512;          // 16 warps per SM at 128 registers: one CTA per SM holds the weights
 constexpr int kMaxIn = 32, kMaxActions = 8, kMaxConvOut = 16;
+constexpr int kMaxInWide = 256;        // input widths 33..256 (search: (2R-1)^2 + 2 obs values + 4 + n) take the wide instantiations
 constexpr int kRowsPerWarp = 4;
 
 // ------------------------------------------------------------------------------------------------
@@ -203,6 +204,8 @@ __device__ __forceinline__ void policy_choose_action(const PolicyParams& p, int 
     p.actions[r] = (uint8_t)act;
 }
 
+// S = 32-wide slices of the input row a lane holds (elements lane + 32 j): 1 for widths <= 32, kMaxInWide / 32 above
+template <int S>
 __global__ void __launch_bounds__(kPolicyThreads, 1) policy_kernel(const __grid_constant__ PolicyParams p) {
     extern __shared__ __align__(16) float wsm[];
     constexpr unsigned FULL = 0xffffffffu;
@@ -228,25 +231,48 @@ __global__ void __launch_bounds__(kPolicyThreads, 1) policy_kernel(const __grid_
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpc = kPolicyThreads / 32;
     for (int rb = (blockIdx.x * wpc + warp) * RPW; rb < p.rows; rb += gridDim.x * wpc * RPW) {
         int row[RPW];
-        float inv[RPW], x0[RPW], x1[RPW], h0[RPW], h1[RPW];
+        float inv[RPW][S], x0[RPW], x1[RPW], h0[RPW], h1[RPW];
 #pragma unroll
         for (int u = 0; u < RPW; ++u) {
             const int r = min(rb + u, p.rows - 1);                      // a short last block repeats its last row (writes are guarded)
             row[u] = r;
-            // input element `lane` (agent/agent.py:38-50)
-            inv[u] = lane < in_dim ? policy_input(p, r, (p.use_last && p.last_action) ? (int)p.last_action[r] : 255, lane) : 0.f;
+            // input elements `lane + 32 j` (agent/agent.py:38-50)
+            if constexpr (S == 1) {
+                inv[u][0] = lane < in_dim ? policy_input(p, r, (p.use_last && p.last_action) ? (int)p.last_action[r] : 255, lane) : 0.f;
+            } else {
+                const int la = (p.use_last && p.last_action) ? (int)p.last_action[r] : 255;
+#pragma unroll
+                for (int j = 0; j < S; ++j) inv[u][j] = lane + 32 * j < in_dim ? policy_input(p, r, la, lane + 32 * j) : 0.f;
+            }
             x0[u] = b1[lane]; x1[u] = b1[lane + 32];
             h0[u] = p.hidden[(size_t)r * kH + lane]; h1[u] = p.hidden[(size_t)r * kH + lane + 32];
         }
         __syncwarp();                                                    // all rows' last actions are read before any is rewritten
-        // fc1 + ReLU: outputs j = lane, lane + 32
-        for (int k = 0; k < in_dim; ++k) {
-            const float w0 = W1T[k * kH + lane], w1 = W1T[k * kH + lane + 32];
+        // fc1 + ReLU: outputs j = lane, lane + 32; k ascending over the whole width
+        if constexpr (S == 1) {
+            for (int k = 0; k < in_dim; ++k) {
+                const float w0 = W1T[k * kH + lane], w1 = W1T[k * kH + lane + 32];
 #pragma unroll
-            for (int u = 0; u < RPW; ++u) {
-                const float v = __shfl_sync(FULL, inv[u], k);
-                x0[u] = fmaf(v, w0, x0[u]);
-                x1[u] = fmaf(v, w1, x1[u]);
+                for (int u = 0; u < RPW; ++u) {
+                    const float v = __shfl_sync(FULL, inv[u][0], k);
+                    x0[u] = fmaf(v, w0, x0[u]);
+                    x1[u] = fmaf(v, w1, x1[u]);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < S; ++j) {
+                const int kend = min(32, in_dim - 32 * j);             // slice j holds elements 32 j .. 32 j + kend - 1
+                for (int kk = 0; kk < kend; ++kk) {
+                    const int k = 32 * j + kk;
+                    const float w0 = W1T[k * kH + lane], w1 = W1T[k * kH + lane + 32];
+#pragma unroll
+                    for (int u = 0; u < RPW; ++u) {
+                        const float v = __shfl_sync(FULL, inv[u][j], kk);
+                        x0[u] = fmaf(v, w0, x0[u]);
+                        x1[u] = fmaf(v, w1, x1[u]);
+                    }
+                }
             }
         }
 #pragma unroll
@@ -334,6 +360,23 @@ void pack_umma(unsigned char* dst, const float* w, int N, int K, int Npad, int K
         for (int n = 0; n < Npad; ++n)
             d[(size_t)(k / 8) * Npad * 8 + (size_t)n * 8 + (k % 8)] = (n < N && k < K) ? host_bf16(w[(size_t)n * K + k]) : (uint16_t)0;
 }
+// the weight block every CTA of policy_tc_kernel<P, K1> copies into shared memory
+template <int K1>
+std::vector<unsigned char> pack_tc(const cs_policy_weights* hw, int in_dim, int A) {
+    using L = cspol::TcLayout<K1>;
+    std::vector<unsigned char> tc((size_t)L::kWeightBytes, 0);
+    pack_umma(tc.data() + L::kOffW1, hw->fc1_w, kH, in_dim, 64, K1);
+    pack_umma(tc.data() + L::kOffWih, hw->w_ih, 3 * kH, kH, 192, 64);
+    pack_umma(tc.data() + L::kOffWhh, hw->w_hh, 3 * kH, kH, 192, 64);
+    pack_umma(tc.data() + L::kOffW2a, hw->fc2a_w, kH, kH, 64, 64);
+    pack_umma(tc.data() + L::kOffW2b, hw->fc2b_w, A, kH, cspol::kTcNq, 64);
+    float* b = reinterpret_cast<float*>(tc.data() + L::kOffBias);
+    for (int j = 0; j < 64; ++j) b[j] = hw->fc1_b[j];
+    for (int j = 0; j < 128; ++j) b[64 + j] = hw->b_ih[j] + hw->b_hh[j];          // r | z gates: the two biases only ever appear summed
+    for (int j = 0; j < 64; ++j) { b[192 + j] = hw->b_ih[128 + j]; b[256 + j] = hw->b_hh[128 + j]; b[320 + j] = hw->fc2a_b[j]; }
+    for (int a = 0; a < A; ++a) b[384 + a] = hw->fc2b_b[a];
+    return tc;
+}
 }  // namespace
 
 struct cs_policy {
@@ -342,7 +385,8 @@ struct cs_policy {
     float* d_conv_w;
     size_t w_floats;
     float* d_w;
-    unsigned char* d_wtc;        // tensor-core weights (packed for every allowed input width, <= kTcK1 = 32)
+    unsigned char* d_wtc;        // tensor-core weights, packed for the instantiation the width selects
+    int wide;                    // input width > kMaxIn: the wide instantiations (policy_kernel<8>, policy_tc_kernel<P, kTcK1Wide>)
 };
 
 extern "C" {
@@ -354,7 +398,7 @@ int cs_policy_create(const cs_policy_cfg* cfg, const cs_policy_weights* hw, cs_p
     CS_REQUIRE(cfg->n_actions >= 1 && cfg->n_actions <= kMaxActions, "cs_policy_create: n_actions must be in 1..%d", kMaxActions);
     CS_REQUIRE(cfg->conv_out_dim >= 0 && cfg->conv_out_dim <= kMaxConvOut, "cs_policy_create: conv_out_dim must be in 0..%d", kMaxConvOut);
     const int in_dim = cfg->conv_out_dim + cfg->obs_dim + (cfg->last_action ? cfg->n_actions : 0) + (cfg->reuse_network ? cfg->n_agents : 0);
-    CS_REQUIRE(cfg->obs_dim >= 1 && in_dim <= kMaxIn, "cs_policy_create: input width %d exceeds %d (the conv front end is not part of this kernel)", in_dim, kMaxIn);
+    CS_REQUIRE(cfg->obs_dim >= 1 && in_dim <= kMaxInWide, "cs_policy_create: input width %d exceeds %d", in_dim, kMaxInWide);
     CS_REQUIRE(hw->fc1_w && hw->fc1_b && hw->w_ih && hw->w_hh && hw->b_ih && hw->b_hh && hw->fc2a_w && hw->fc2a_b && hw->fc2b_w && hw->fc2b_b,
                "cs_policy_create: null weight pointer");
     const int A = cfg->n_actions;
@@ -377,29 +421,27 @@ int cs_policy_create(const cs_policy_cfg* cfg, const cs_policy_weights* hw, cs_p
     h->device = cfg->device; h->obs_dim = cfg->obs_dim; h->n_actions = A; h->n_agents = cfg->n_agents;
     h->use_last = cfg->last_action; h->use_id = cfg->reuse_network; h->in_dim = in_dim; h->w_floats = pk.size(); h->d_w = nullptr;
     h->feat_dim = cfg->conv_out_dim; h->d_conv_w = nullptr; memset(&h->conv, 0, sizeof(h->conv));
+    h->wide = in_dim > kMaxIn;
     cudaError_t e = cudaSetDevice(cfg->device);
     if (e == cudaSuccess) e = cudaMalloc(&h->d_w, pk.size() * sizeof(float));
     if (e == cudaSuccess) e = cudaMemcpy(h->d_w, pk.data(), pk.size() * sizeof(float), cudaMemcpyHostToDevice);
     // the largest weight block any policy can have, so that handles of different widths coexist
     constexpr size_t kMaxWeights = (size_t)kMaxIn * kH + kH + 2 * (kH * 3 * kH + 3 * kH) + kH * kH + kH + kMaxActions * kH + kMaxActions;
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kMaxWeights * sizeof(float)));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kMaxWeights * sizeof(float)));
+    // the wide instantiation's own limit (184 KB at width 256 and 8 actions)
+    constexpr size_t kMaxWeightsWide = kMaxWeights + (size_t)(kMaxInWide - kMaxIn) * kH;
+    if (e == cudaSuccess && h->wide)
+        e = cudaFuncSetAttribute(policy_kernel<kMaxInWide / 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kMaxWeightsWide * sizeof(float)));
     h->d_wtc = nullptr;
-    if (e == cudaSuccess && in_dim <= cspol::kTcK1) {
+    if (e == cudaSuccess) {
         using namespace cspol;
-        std::vector<unsigned char> tc((size_t)kTcWeightBytes, 0);
-        pack_umma(tc.data() + kOffW1, hw->fc1_w, kH, in_dim, 64, kTcK1);
-        pack_umma(tc.data() + kOffWih, hw->w_ih, 3 * kH, kH, 192, 64);
-        pack_umma(tc.data() + kOffWhh, hw->w_hh, 3 * kH, kH, 192, 64);
-        pack_umma(tc.data() + kOffW2a, hw->fc2a_w, kH, kH, 64, 64);
-        pack_umma(tc.data() + kOffW2b, hw->fc2b_w, A, kH, kTcNq, 64);
-        float* b = reinterpret_cast<float*>(tc.data() + kOffBias);
-        for (int j = 0; j < 64; ++j) b[j] = hw->fc1_b[j];
-        for (int j = 0; j < 128; ++j) b[64 + j] = hw->b_ih[j] + hw->b_hh[j];          // r | z gates: the two biases only ever appear summed
-        for (int j = 0; j < 64; ++j) { b[192 + j] = hw->b_ih[128 + j]; b[256 + j] = hw->b_hh[128 + j]; b[320 + j] = hw->fc2a_b[j]; }
-        for (int a = 0; a < A; ++a) b[384 + a] = hw->fc2b_b[a];
+        const std::vector<unsigned char> tc = h->wide ? pack_tc<kTcK1Wide>(hw, in_dim, A) : pack_tc<kTcK1>(hw, in_dim, A);
         e = cudaMalloc(&h->d_wtc, tc.size());
         if (e == cudaSuccess) e = cudaMemcpy(h->d_wtc, tc.data(), tc.size(), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(cspol::policy_tc_kernel<PolicyParams>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemBytes);
+        if (e == cudaSuccess && !h->wide)
+            e = cudaFuncSetAttribute(policy_tc_kernel<PolicyParams, kTcK1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcLayout<kTcK1>::kSmemBytes);
+        if (e == cudaSuccess && h->wide)
+            e = cudaFuncSetAttribute(policy_tc_kernel<PolicyParams, kTcK1Wide>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcLayout<kTcK1Wide>::kSmemBytes);
     }
     if (e != cudaSuccess) { cudaFree(h->d_w); cudaFree(h->d_wtc); delete h; }
     CS_CUDA(e);
@@ -426,14 +468,21 @@ int cs_policy_act(cs_policy* h, const cs_policy_io* io, void* stream) {
     CS_REQUIRE(h->feat_dim == 0 || io->feat, "cs_policy_act: this policy has a conv front end: io.feat (cs_policy_conv_features) is required");
     CS_REQUIRE(io->mode == 0 || io->mode == 1, "cs_policy_act: mode must be 0 (argmax / epsilon-greedy) or 1 (softmax sampling)");
     CS_REQUIRE(io->precision == 0 || io->precision == 1, "cs_policy_act: precision must be 0 (fp32) or 1 (bf16 tensor cores)");
-    CS_REQUIRE(io->precision == 0 || h->d_wtc, "cs_policy_act: the tensor-core kernel needs an input width <= %d", cspol::kTcK1);
+    CS_REQUIRE(io->precision == 0 || h->d_wtc, "cs_policy_act: this policy has no tensor-core weights");
     p.w = h->d_w; p.obs = io->obs; p.last_action = io->last_action; p.avail = io->avail; p.hidden = io->hidden; p.q = io->q;
     p.actions = io->actions;
     if (io->precision == 1) {
-        // tensor cores: one 128-row tile per CTA iteration, two CTAs per SM (each holds its own copy of the weights)
-        const int tiles = (io->rows + cspol::kTcRows - 1) / cspol::kTcRows;
-        const int grid_tc = tiles < 2 * CS_NUM_SMS_B200 ? tiles : 2 * CS_NUM_SMS_B200;
-        cspol::policy_tc_kernel<PolicyParams><<<grid_tc, cspol::kTcThreads, cspol::kTcSmemBytes, (cudaStream_t)stream>>>(p);
+        // tensor cores: one 128-row tile per CTA iteration, two CTAs per SM (each holds its own copy of the weights); the
+        // wide instantiation, one CTA per SM
+        using namespace cspol;
+        const int tiles = (io->rows + kTcRows - 1) / kTcRows;
+        if (h->wide) {
+            const int grid_tc = tiles < CS_NUM_SMS_B200 ? tiles : CS_NUM_SMS_B200;
+            policy_tc_kernel<PolicyParams, kTcK1Wide><<<grid_tc, kTcThreads, TcLayout<kTcK1Wide>::kSmemBytes, (cudaStream_t)stream>>>(p);
+        } else {
+            const int grid_tc = tiles < 2 * CS_NUM_SMS_B200 ? tiles : 2 * CS_NUM_SMS_B200;
+            policy_tc_kernel<PolicyParams, kTcK1><<<grid_tc, kTcThreads, TcLayout<kTcK1>::kSmemBytes, (cudaStream_t)stream>>>(p);
+        }
         cs_count_launch(1);
         CS_CUDA(cudaGetLastError());
         return CS_OK;
@@ -441,7 +490,10 @@ int cs_policy_act(cs_policy* h, const cs_policy_io* io, void* stream) {
     const int wpc = (kPolicyThreads / 32) * kRowsPerWarp;
     int grid = (io->rows + wpc - 1) / wpc;
     if (grid > CS_NUM_SMS_B200) grid = CS_NUM_SMS_B200;                   // persistent: one CTA per SM keeps the weights resident
-    policy_kernel<<<grid, kPolicyThreads, h->w_floats * sizeof(float), (cudaStream_t)stream>>>(p);
+    if (h->wide)
+        policy_kernel<kMaxInWide / 32><<<grid, kPolicyThreads, h->w_floats * sizeof(float), (cudaStream_t)stream>>>(p);
+    else
+        policy_kernel<1><<<grid, kPolicyThreads, h->w_floats * sizeof(float), (cudaStream_t)stream>>>(p);
     cs_count_launch(1);
     CS_CUDA(cudaGetLastError());
     return CS_OK;

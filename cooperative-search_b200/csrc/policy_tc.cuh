@@ -1,7 +1,7 @@
 // Agent network on the 5th-generation tensor cores (tcgen05 + TMEM), included by policy.cu.
 //
 // RNN.forward (network/base_net.py:30-47) for a tile of 128 (env, agent) rows is five small GEMMs with a shared M = 128:
-//   fc1   [128 x 32] x [32 -> 64]                       -> +b, ReLU           -> x1     (input width <= 32, zero padded)
+//   fc1   [128 x K1] x [K1 -> 64]                       -> +b, ReLU           -> x1     (input width zero padded to K1)
 //   GRU   [128 x 64] x W_ih^T and [128 x 64] x W_hh^T   -> gates r | z | n    -> h'     (network/base_net.py:43, torch GRUCell)
 //   fc2.0 [128 x 64] x [64 -> 64]                       -> +b, ReLU           -> f
 //   fc2.2 [128 x 64] x [64 -> A (padded to 16)]         -> +b                 -> q
@@ -17,6 +17,9 @@
 // epilogue: bias, ReLU / sigmoid / tanh, the GRU blend, the bf16 operand of the next GEMM, and finally the masked
 // argmax / epsilon-greedy / softmax-sampling action choice of agent/agent.py:66-97.  The r and z gates accumulate
 // x1 W_ir^T + h W_hr^T in the same TMEM columns.  bf16 operands, fp32 accumulation, fp32 hidden state in HBM.
+// Two instantiations: K1 = 32 for input widths <= 32 (two CTAs per SM) and K1 = 256 for widths 33..256, e.g. the
+// search agents (171 obs values + 4 + n): one CTA per SM, fc1 issues only ceil(width / 16) K-steps, and the obs rows
+// of a tile are staged by the whole CTA with coalesced loads (tc_wide_inputs).
 #pragma once
 #include <cuda_bf16.h>
 
@@ -24,24 +27,30 @@ namespace cspol {
 
 constexpr int kTcThreads = 256;                    // two threads per row
 constexpr int kTcRows = 128;                       // rows per tile = UMMA M
-constexpr int kTcK1 = 32;                          // fc1 input width, padded
+constexpr int kTcK1 = 32;                          // fc1 input width, padded (input widths <= 32)
+constexpr int kTcK1Wide = 256;                     // fc1 input width, padded, of the wide instantiation (widths 33..256)
 constexpr int kTcNq = 16;                          // action-value width, padded (UMMA N is a multiple of 16)
 constexpr int kTcTmemCols = 256;
 constexpr int kALbo = (kTcRows + 1) * 16;          // bytes between K chunks of an A operand (129 rows: bank-conflict-free transposes)
-// shared-memory map (bytes)
-constexpr int kOffW1 = 0;                                   // [4 chunks][64][8] bf16
-constexpr int kOffWih = kOffW1 + (kTcK1 / 8) * 64 * 16;     // [8][192][8]
-constexpr int kOffWhh = kOffWih + 8 * 192 * 16;
-constexpr int kOffW2a = kOffWhh + 8 * 192 * 16;             // [8][64][8]
-constexpr int kOffW2b = kOffW2a + 8 * 64 * 16;              // [8][16][8]
-constexpr int kOffBias = kOffW2b + 8 * kTcNq * 16;          // fp32: b1[64] | b_rz[128] | b_in[64] | b_hn[64] | b2a[64] | b2b[16]
-constexpr int kBiasFloats = 64 + 128 + 64 + 64 + 64 + kTcNq;
-constexpr int kTcWeightBytes = kOffBias + kBiasFloats * 4;  // what the host packs and every CTA copies
-constexpr int kOffA0 = (kTcWeightBytes + 127) & ~127;       // [4][129 rows][8] bf16
-constexpr int kOffAX = kOffA0 + (kTcK1 / 8) * kALbo;        // [8][129][8]: x1, later f
-constexpr int kOffAH = kOffAX + 8 * kALbo;                  // [8][129][8]: h, later h'
-constexpr int kOffBar = kOffAH + 8 * kALbo;                 // mbarrier (8 B) + TMEM base address (4 B)
-constexpr int kTcSmemBytes = kOffBar + 16;
+// shared-memory map (bytes) of the instantiation with padded fc1 width K1
+template <int K1>
+struct TcLayout {
+    static constexpr int kOffW1 = 0;                                   // [K1/8 chunks][64][8] bf16
+    static constexpr int kOffWih = kOffW1 + (K1 / 8) * 64 * 16;        // [8][192][8]
+    static constexpr int kOffWhh = kOffWih + 8 * 192 * 16;
+    static constexpr int kOffW2a = kOffWhh + 8 * 192 * 16;             // [8][64][8]
+    static constexpr int kOffW2b = kOffW2a + 8 * 64 * 16;              // [8][16][8]
+    static constexpr int kOffBias = kOffW2b + 8 * kTcNq * 16;          // fp32: b1[64] | b_rz[128] | b_in[64] | b_hn[64] | b2a[64] | b2b[16]
+    static constexpr int kBiasFloats = 64 + 128 + 64 + 64 + 64 + kTcNq;
+    static constexpr int kWeightBytes = kOffBias + kBiasFloats * 4;    // what the host packs and every CTA copies
+    static constexpr int kOffA0 = (kWeightBytes + 127) & ~127;         // [K1/8][129 rows][8] bf16
+    static constexpr int kOffAX = kOffA0 + (K1 / 8) * kALbo;           // [8][129][8]: x1, later f
+    static constexpr int kOffAH = kOffAX + 8 * kALbo;                  // [8][129][8]: h, later h'
+    static constexpr int kOffBar = kOffAH + 8 * kALbo;                 // mbarrier (8 B) + TMEM base address (4 B)
+    static constexpr int kSmemBytes = kOffBar + 16;
+    static constexpr int kCtasPerSm = K1 == kTcK1 ? 2 : 1;             // 2 x 104 KB, or 1 x 188 KB of the 227 KB
+};
+static_assert(TcLayout<kTcK1Wide>::kSmemBytes <= 227 * 1024, "the wide instantiation must fit one CTA's shared memory");
 
 __device__ __forceinline__ uint32_t tc_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -117,15 +126,86 @@ __device__ __forceinline__ void tc_operands_ready() {
     __syncthreads();
 }
 
-template <class P>
-__global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_constant__ P p) {
+// fc1 input rows of one tile for the wide instantiation (widths 33..256), as bf16 in A0's chunks 0 .. 2 * ksteps - 1.
+// A search row is 171 floats (684 B), so a thread that assembled its own row with scalar loads would touch 32 lines
+// per warp load.  Instead the tile's obs rows, one contiguous block of rows * obs_dim floats, are read by the whole CTA
+// with coalesced 16-byte loads and scattered element by element into A0; each thread then writes what is not obs in
+// its own row (conv features, the one-hot blocks, which are generated, not loaded, and the zero padding up to the
+// last K-step).  The two writers never share a 16-byte chunk except at the edges of the obs range, where both use
+// 2-byte stores.
+template <class L, class P>
+__device__ __forceinline__ void tc_wide_inputs(const P& p, unsigned char* sm, int tile, int r, int half, int tid, int ksteps) {
+    constexpr int kU = 8;                                              // 16-byte loads in flight per thread
+    const int F = p.feat_dim, D = p.obs_dim, A = p.n_actions;
+    unsigned char* a0 = sm + L::kOffA0;
+    auto put = [&](int rw, int k, float v) {
+        *reinterpret_cast<__nv_bfloat16*>(a0 + (k >> 3) * kALbo + rw * 16 + (k & 7) * 2) = __float2bfloat16_rn(v);
+    };
+    // this thread's row: everything but the obs elements
+    {
+        const int rw = tid & (kTcRows - 1);                            // (r: a dead row of a last tile repeats the last row)
+        const int la = (p.use_last && p.last_action) ? (int)p.last_action[r] : 255;
+        const int kla = (p.use_last && la < A) ? F + D + la : -1;
+        const int kid = p.use_id ? F + D + (p.use_last ? A : 0) + r % p.n_agents : -1;
+        for (int c = half; c < 2 * ksteps; c += 2) {
+            const int k0 = 8 * c;
+            float x[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const int k = k0 + i;
+                x[i] = k < F ? p.feat[(size_t)(r / p.n_agents) * F + k] : ((k == kla || k == kid) ? 1.f : 0.f);
+            }
+            if (k0 + 8 <= F || k0 >= F + D) {
+                *reinterpret_cast<uint4*>(a0 + c * kALbo + rw * 16) = tc_pack8(x);
+            } else if (k0 < F || k0 + 8 > F + D) {
+#pragma unroll
+                for (int i = 0; i < 8; ++i)
+                    if (k0 + i < F || k0 + i >= F + D) put(rw, k0 + i, x[i]);
+            }
+        }
+    }
+    // the tile's obs block: element e is obs[row0 + e / D][e % D] -> A0 (row e / D, k = F + e % D)
+    const int nrows = p.rows - tile * kTcRows < kTcRows ? p.rows - tile * kTcRows : kTcRows;
+    const float* blk = p.obs + (size_t)tile * kTcRows * D;
+    const int n = nrows * D;
+    int head = (int)(((16u - ((uint32_t)(uintptr_t)blk & 15u)) & 15u) >> 2);   // scalar elements before the first 16-byte boundary
+    head = head < n ? head : n;
+    auto put_run = [&](int e, const float* v, int cnt) {
+        int rw = e / D, k = e - rw * D;
+        for (int j = 0; j < cnt; ++j) {
+            put(rw, F + k, v[j]);
+            if (++k == D) { k = 0; ++rw; }
+        }
+    };
+    if (tid < head) { const float v = __ldcs(blk + tid); put_run(tid, &v, 1); }
+    const float4* b4 = reinterpret_cast<const float4*>(blk + head);
+    const int n4 = (n - head) >> 2;
+    for (int i0 = tid; i0 < n4; i0 += kU * kTcThreads) {
+        float4 v[kU];
+#pragma unroll
+        for (int u = 0; u < kU; ++u)
+            if (i0 + u * kTcThreads < n4) v[u] = __ldcs(b4 + i0 + u * kTcThreads);
+#pragma unroll
+        for (int u = 0; u < kU; ++u)
+            if (i0 + u * kTcThreads < n4) {
+                const float w[4] = {v[u].x, v[u].y, v[u].z, v[u].w};
+                put_run(head + 4 * (i0 + u * kTcThreads), w, 4);
+            }
+    }
+    const int t0 = head + 4 * n4;
+    if (t0 + tid < n) { const float v = __ldcs(blk + t0 + tid); put_run(t0 + tid, &v, 1); }
+}
+
+template <class P, int K1>
+__global__ void __launch_bounds__(kTcThreads, TcLayout<K1>::kCtasPerSm) policy_tc_kernel(const __grid_constant__ P p) {
+    using L = TcLayout<K1>;
     extern __shared__ __align__(128) unsigned char sm[];
     const int tid = threadIdx.x, warp = tid >> 5;
     const int row = tid & (kTcRows - 1), half = tid >> 7;             // this thread's row of the tile and its half of the columns
     const uint32_t sbase = tc_smem_u32(sm);
-    const uint32_t bar = sbase + kOffBar;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + kOffBar + 8);
-    const float* bias = reinterpret_cast<const float*>(sm + kOffBias);
+    const uint32_t bar = sbase + L::kOffBar;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + L::kOffBar + 8);
+    const float* bias = reinterpret_cast<const float*>(sm + L::kOffBias);
     const float *b1 = bias, *b_rz = bias + 64, *b_in = bias + 192, *b_hn = bias + 256, *b2a = bias + 320, *b2b = bias + 384;
     const int A = p.n_actions;
 
@@ -133,7 +213,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
     {
         const uint4* src = reinterpret_cast<const uint4*>(p.wtc);
         uint4* dst = reinterpret_cast<uint4*>(sm);
-        for (int i = tid; i < kTcWeightBytes / 16; i += kTcThreads) dst[i] = __ldg(src + i);
+        for (int i = tid; i < L::kWeightBytes / 16; i += kTcThreads) dst[i] = __ldg(src + i);
     }
     if (tid == 0) {
         asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
@@ -149,17 +229,18 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
     const uint32_t trow = tmem + ((uint32_t)((warp & 3) * 32) << 16);  // this warp's 32 TMEM lanes
     uint32_t phase = 0;
 
-    unsigned char* myA0 = sm + kOffA0 + row * 16;
-    unsigned char* myAX = sm + kOffAX + row * 16;
-    unsigned char* myAH = sm + kOffAH + row * 16;
+    unsigned char* myA0 = sm + L::kOffA0 + row * 16;
+    unsigned char* myAX = sm + L::kOffAX + row * 16;
+    unsigned char* myAH = sm + L::kOffAH + row * 16;
 
+    const int ksteps1 = K1 == kTcK1 ? kTcK1 / 16 : (p.in_dim + 15) >> 4;   // fc1 K-steps: the wide form issues only those the width needs
     for (int tile = blockIdx.x; tile * kTcRows < p.rows; tile += gridDim.x) {
         const int r_raw = tile * kTcRows + row;
         const bool live = r_raw < p.rows;
         const int r = live ? r_raw : p.rows - 1;
         // ---- inputs: [conv features of the env's map ||] obs || last-action one-hot || agent-id one-hot
         //      (network/base_net.py:31-41, agent/agent.py:38-50)
-        {
+        if constexpr (K1 == kTcK1) {
             const int la = (p.use_last && p.last_action) ? (int)p.last_action[r] : 255;
 #pragma unroll
             for (int cc = 0; cc < kTcK1 / 16; ++cc) {
@@ -169,12 +250,14 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
                 for (int i = 0; i < 8; ++i) x[i] = policy_input(p, r, la, 8 * c + i);
                 *reinterpret_cast<uint4*>(myA0 + c * kALbo) = tc_pack8(x);
             }
+        } else {
+            tc_wide_inputs<L>(p, sm, tile, r, half, tid, ksteps1);
         }
         tc_operands_ready();
         // ---- fc1
         if (tid == 0) {
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            tc_gemm(tmem + 0, sbase + kOffA0, sbase + kOffW1, 64, 0, 64, kTcK1 / 16, false);
+            tc_gemm(tmem + 0, sbase + L::kOffA0, sbase + L::kOffW1, 64, 0, 64, ksteps1, false);
             tc_commit(bar);
         }
         // ... and while the tensor core works on fc1: this thread's half of the row's hidden state (units 32 * half ...), read
@@ -193,7 +276,16 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
             const long long rn = (long long)(tile + (int)gridDim.x) * kTcRows + row;
             if (rn < p.rows) {
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(p.hidden + (size_t)rn * 64 + 32 * half));
-                if (half == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.obs + (size_t)rn * p.obs_dim));
+                if (K1 == kTcK1 && half == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.obs + (size_t)rn * p.obs_dim));
+            }
+            if constexpr (K1 != kTcK1) {                               // the next tile's obs block, 128-byte lines spread over the CTA
+                const long long r0 = (long long)(tile + (int)gridDim.x) * kTcRows;
+                if (r0 < p.rows) {
+                    const long long nrows = p.rows - r0 < kTcRows ? p.rows - r0 : kTcRows;
+                    const char* blk = reinterpret_cast<const char*>(p.obs + (size_t)r0 * p.obs_dim);
+                    const long long bytes = nrows * p.obs_dim * 4;
+                    for (long long o = 128ll * tid; o < bytes; o += 128ll * kTcThreads) asm volatile("prefetch.global.L2 [%0];" ::"l"(blk + o));
+                }
             }
         }
         tc_wait(bar, phase); phase ^= 1u;
@@ -213,10 +305,10 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
         // ---- GRU gates: r | z accumulate x1 W_i^T + h W_h^T in columns 0..127; n keeps its two halves apart
         if (tid == 0) {
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            tc_gemm(tmem + 0, sbase + kOffAX, sbase + kOffWih, 192, 0, 128, 4, false);
-            tc_gemm(tmem + 0, sbase + kOffAH, sbase + kOffWhh, 192, 0, 128, 4, true);
-            tc_gemm(tmem + 128, sbase + kOffAX, sbase + kOffWih, 192, 128, 64, 4, false);
-            tc_gemm(tmem + 192, sbase + kOffAH, sbase + kOffWhh, 192, 128, 64, 4, false);
+            tc_gemm(tmem + 0, sbase + L::kOffAX, sbase + L::kOffWih, 192, 0, 128, 4, false);
+            tc_gemm(tmem + 0, sbase + L::kOffAH, sbase + L::kOffWhh, 192, 0, 128, 4, true);
+            tc_gemm(tmem + 128, sbase + L::kOffAX, sbase + L::kOffWih, 192, 128, 64, 4, false);
+            tc_gemm(tmem + 192, sbase + L::kOffAH, sbase + L::kOffWhh, 192, 128, 64, 4, false);
             tc_commit(bar);
         }
         tc_wait(bar, phase); phase ^= 1u;
@@ -251,7 +343,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
         // ---- fc2.0
         if (tid == 0) {
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            tc_gemm(tmem + 0, sbase + kOffAH, sbase + kOffW2a, 64, 0, 64, 4, false);
+            tc_gemm(tmem + 0, sbase + L::kOffAH, sbase + L::kOffW2a, 64, 0, 64, 4, false);
             tc_commit(bar);
         }
         tc_wait(bar, phase); phase ^= 1u;
@@ -271,7 +363,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const __grid_c
         // ---- fc2.2 -> action values
         if (tid == 0) {
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            tc_gemm(tmem + 64, sbase + kOffAX, sbase + kOffW2b, kTcNq, 0, kTcNq, 4, false);
+            tc_gemm(tmem + 64, sbase + L::kOffAX, sbase + L::kOffW2b, kTcNq, 0, kTcNq, 4, false);
             tc_commit(bar);
         }
         tc_wait(bar, phase); phase ^= 1u;

@@ -2,10 +2,11 @@
 action choice of Agents.choose_action (agent/agent.py:33-97) for every (env, agent) row of a vectorised env at once,
 in one kernel launch (csrc/policy.cu, csrc/policy_tc.cuh).  The reference evaluates one (1, in) row per agent per step.
 
-precision "bf16" (the default, for every allowed input width up to 32): the five GEMMs of a 128-row tile run on the
-tcgen05 tensor cores with bf16 operands, fp32 accumulators in tensor memory and an fp32 hidden state; "fp32": the
-CUDA-core kernel that equals the reference's torch modules to 1e-5.  Both are held to a float64 reference with
-per-element error bounds (oracle/policy_ref.py, tests/test_gpu_policy_reference.py).
+precision "bf16" (the default): the five GEMMs of a 128-row tile run on the tcgen05 tensor cores with bf16 operands,
+fp32 accumulators in tensor memory and an fp32 hidden state; "fp32": the CUDA-core kernel that equals the reference's
+torch modules to 1e-5.  Input widths up to 256: each kernel has one instantiation for widths <= 32 (the flight agents)
+and one for 33..256 (the search agents: (2R-1)^2 + 2 obs values + 4 + n_agents, 239 at 64 agents), chosen by width.
+Both are held to a float64 reference with per-element error bounds (oracle/policy_ref.py, tests/test_gpu_policy_reference.py).
 alg: "q" = masked argmax / epsilon-greedy (qmix, vdn; dop's actor is the same network class with the actor's weights),
 "reinforce" = softmax sampling (agent/agent.py:77-97)."""
 import ctypes as C
@@ -92,17 +93,22 @@ class BatchedRNNAgents:
         if alg not in ("q", "reinforce"):
             raise CoopSearchError("alg must be 'q' (argmax / epsilon-greedy) or 'reinforce' (softmax sampling)")
         self.precision, self.alg = precision, alg
-        self.kernel_name = "policy_tc_kernel (tcgen05.mma, bf16 operands, TMEM accumulators)" if precision == "bf16" else "policy_kernel (fp32, CUDA cores)"
+        if precision == "bf16":
+            self.kernel_name = "policy_tc_kernel<K1=%d> (tcgen05.mma, bf16 operands, TMEM accumulators)" % (32 if in_dim <= 32 else 256)
+        else:
+            self.kernel_name = "policy_kernel<S=%d> (fp32, CUDA cores)" % (1 if in_dim <= 32 else 8)
 
     def init_hidden(self, mask=None):
-        """policy.init_hidden(1) + last_action = zeros (rollout.py:31-33) for all envs, or those with mask[e] != 0."""
+        """policy.init_hidden(1) + last_action = zeros (rollout.py:31-33) for all envs, or those with mask[e] != 0.
+        A device mask (e.g. the terminated flags of an auto-resetting env) is applied without a host synchronisation,
+        so the call can be captured in a CUDA graph."""
         if mask is None:
             self.hidden.zero_()
             self.actions.fill_(255)
         else:
             m = torch.as_tensor(mask, device=self.device).bool()
-            self.hidden[m] = 0
-            self.actions[m] = 255
+            self.hidden.masked_fill_(m.reshape(m.shape + (1,) * (self.hidden.dim() - m.dim())), 0)
+            self.actions.masked_fill_(m.reshape(m.shape + (1,) * (self.actions.dim() - m.dim())), 255)
 
     def conv_features(self, env=None, prob_map_tiles=None):
         """The conv features of every env's belief map ([E, conv_out_dim], also kept as ``self.feat``), read once per env

@@ -426,13 +426,14 @@ typedef struct cs_policy_io {          /* DEVICE pointers; row r = env r / n_age
     float* q;                          /* [rows][n_actions] out or NULL                                   */
     uint8_t* actions;                  /* [rows] out; may be the same buffer as last_action               */
     int32_t precision;                 /* 0 = fp32 on CUDA cores; 1 = bf16 operands on the tcgen05 tensor cores,
-                                          fp32 accumulation and hidden state (input width <= 16)          */
+                                          fp32 accumulation and hidden state (both: input width <= 256)   */
     int32_t mode;                      /* 0 = masked argmax / epsilon-greedy (agent.py:66-75);
                                           1 = softmax sampling of alg=reinforce (agent.py:77-97)            */
     const float* feat;                 /* [rows / n_agents][conv_out_dim] from cs_policy_conv_features, or NULL  */
 } cs_policy_io;
 typedef struct cs_policy cs_policy;
-/* RNN(input_shape, args) + load_state_dict (policy/qmix.py:40-59) */
+/* RNN(input_shape, args) + load_state_dict (policy/qmix.py:40-59).  The fc1 input width (conv_out_dim + obs_dim
+ * [+ n_actions] [+ n_agents]) may be up to 256; larger widths return CS_ERR_INVALID. */
 int cs_policy_create(const cs_policy_cfg* cfg, const cs_policy_weights* host_weights, cs_policy** out);
 void cs_policy_destroy(cs_policy* policy);
 /* Agents.choose_action for every (env, agent) row at once (agent/agent.py:33-97, alg != random) */
