@@ -35,7 +35,8 @@ struct FlightParams {
     int rec, yaw_off, meta_off, state_len;
     long long dyn_rs, dyn_es, tgt_rs, tgt_es;   // strides (in doubles) of a row / an env in dyn and tgt
     int state_stride;            // floats per state row in HBM (state_len rounded up to a multiple of 4)
-    int s_lut, s_warp;           // lane-per-agent kernel: per-warp shared-memory scratch (doubles) for the heading-table index
+    int pad_[2];                 // keeps the fields below at their 16-byte offsets: ptxas pairs aligned neighbours into one
+                                 // 128-bit constant load, and an 8-byte shift re-pairs them and changes the kernels' code
     int span_cap, span_shift;    // power of two >= 2R: corner rows per agent in the interval pass (and its log2)
     // belief map, stored as 4x4-cell tiles of 64 bytes: cell (i, j) of env e lives at
     // prob_map[e*map_stride + ((i>>2)*tiles + (j>>2))*16 + (i&3)*4 + (j&3)], tiles = ceil(M/4) per side
@@ -159,18 +160,14 @@ static __device__ __noinline__ double2 offlattice_sincos(double h) {
 }
 
 // (sin, cos) of heading h
-__device__ __forceinline__ double2 heading_sincos(const FlightParams& p, const longlong2* lutm, double h) {
+__device__ __forceinline__ double2 heading_sincos(const FlightParams& p, double h) {
     const int k = __double2int_rn(h * p.inv_turn);
     if (k == 0 && fabs(h) < 7.450580596923828e-09) return make_double2(h, 1.0);   // |h| < 2^-27: libm returns sin = h, cos = 1
     if (k >= 1 && k <= 36) {
-#ifdef CS_LUTM_STAGED
-        const longlong2 mt = lutm[k];                      // cluster index staged in shared memory by the CTA
-#else
         // the 37-entry cluster index straight from L1 (every warp of the SM reads the same 592 bytes).  Staging it in shared
         // memory per CTA costs 37 loads and a block barrier before the first state load: measured +2..3 % on the grouped
         // c2 launch and on c3 without it, -1 % on the 1M-env launch.
         const longlong2 mt = __ldg(p.lut_meta + k);
-#endif
         const long long off = __double_as_longlong(h) - mt.x;
         const long long half = mt.y >> 32;
         if (off >= -half && off <= half) return __ldg(p.lut + ((mt.y & 0xffffffffLL) + half + off));

@@ -319,13 +319,7 @@ int cs_flight_create(const cs_flight_cfg* cfg, cs_flight** out) {
     // per env and 4 threads per env match the lane-per-agent kernel's latency
     h->tpe_k = p.E >= 32768 ? 1 : 4;
     if (cfg->lanes_per_env == 1 || cfg->lanes_per_env == 4) h->tpe_k = cfg->lanes_per_env;
-    if (const char* kenv = getenv("CS_TPE_K")) {                               // tuning sweeps only
-        const int kv = atoi(kenv);
-        if (kv == 1 || kv == 4) h->tpe_k = kv;
-    }
     if (h->fused) h->tpe_k = fused_lanes_part0();
-    p.s_lut = 0;
-    p.s_warp = 76;                                        // 37 x 16 B heading-table index, padded
     {
         // belief map geometry: 4x4-cell tiles; scratch of the fused kernel (bytes per env) and of the generic kernel
         // (8-byte words per warp)
@@ -347,7 +341,6 @@ int cs_flight_create(const cs_flight_cfg* cfg, cs_flight** out) {
         h->map_grid = (p.E + per_cta - 1) / per_cta;
         p.pre_stride = up2(2 * n + (m + 2) / 2);
     }
-    h->smem_bytes = (size_t)(kThreads / 32) * p.s_warp * sizeof(double);
     const int env_per_cta = (kThreads / 32) * (32 / h->lpe);
     h->grid = (p.E + env_per_cta - 1) / env_per_cta;
     // structure of arrays exactly where one thread owns one env (flight_tpe_kernel<N, 1>), records otherwise
@@ -357,9 +350,8 @@ int cs_flight_create(const cs_flight_cfg* cfg, cs_flight** out) {
     h->last_map = -1;
 
     int rc = CS_OK;
-    {
-        cudaError_t e = lpa_set_smem_limit(h->smem_bytes);
-        if (e == cudaSuccess && cfg->variant) e = map_set_smem_limit(h->map_smem);
+    if (cfg->variant) {
+        const cudaError_t e = map_set_smem_limit(h->map_smem);
         if (e != cudaSuccess) { cs_set_error("cudaFuncSetAttribute -> %s", cudaGetErrorString(e)); rc = CS_ERR_CUDA; }
     }
     if (rc == CS_OK) rc = flight_alloc(h);
@@ -593,9 +585,6 @@ int cs_flight_group_create(cs_flight* const* envs, int32_t count, cs_flight_grou
         const long long threads = (long long)h->p.E * h->tpe_k;
         const int gx = (int)((threads + kTpeThreads - 1) / kTpeThreads);
         if (gx > g->grid_x) g->grid_x = gx;
-        if (h->p.E > g->max_E) g->max_E = h->p.E;
-        if (i == 0) g->all_even = true;
-        if (h->p.E % 2) g->all_even = false;
         g->envs[i] = h;
         GroupEntry& t = g->table.h[i];
         const FlightParams& p = h->p;

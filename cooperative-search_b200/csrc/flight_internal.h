@@ -41,7 +41,7 @@ struct cs_flight {
     cudaEvent_t ev_step;
     struct MapEvent { cudaEvent_t ev; unsigned long long capture_id; bool valid; } ev_map[2];
     int last_map;         // index into ev_map of the latest map launch, -1 = none
-    size_t smem_bytes, map_smem;
+    size_t map_smem;
     int grid, map_grid;
     uint32_t seq;         // generic map path: value of CS_META_SENSE >> 1 that marks "sensed by the latest call" (constant: launches captured in CUDA graphs replay it)
     double* d_tmpl;
@@ -70,8 +70,6 @@ struct GroupActions { const uint8_t* a[kMaxGroup]; };
 
 struct cs_flight_group {
     int count, n, k, grid_x, device;
-    int max_E;            // the largest handle's num_envs
-    bool all_even;        // every handle has an even num_envs (what the streaming step kernel needs)
     cs_flight* envs[kMaxGroup];
     GroupTable table;
 };
@@ -115,7 +113,6 @@ int fused_lanes_part0();
 
 // flight_lpa.cu: lane-per-agent step / reset kernel (+ the generic belief-map kernel of the flight variant)
 cudaError_t launch_lpa(cs_flight*, int mode, const uint8_t* actions, const uint8_t* mask, uint32_t rflags, cudaStream_t);
-cudaError_t lpa_set_smem_limit(size_t step_bytes);
 
 // flight_mapk.cu: belief-map kernels that run as their own launch
 cudaError_t launch_map_tile(cs_flight*, cudaStream_t);

@@ -8,8 +8,7 @@ namespace {
 // ------------------------------------------------------------------------------------------------
 // The step / reset kernel.  A group of LPE lanes (LPE = power of two >= max(n_agents, target_num)) owns one env:
 // lane a < n holds agent a (x, y, heading, cos, sin) and lane j < m holds target j, all in REGISTERS; positions
-// travel between lanes by warp shuffles.  Every global load is issued up front; nothing is staged through shared
-// memory except the heading-table index (per warp) and the scratch of the warp-wide belief-map pass.
+// travel between lanes by warp shuffles.  Every global load is issued up front; the kernel uses no shared memory.
 // Every warp collective uses the FULL mask and sits in warp-uniform control flow (groups are told apart by
 // predicates, not branches), so no partial-mask MATCH/REDUX sequences or divergence barriers are generated.
 //   pass 0 (STEP): _agent_step -> _update_obs -> step bookkeeping            (flight_env_easy.py:255-314)
@@ -22,14 +21,11 @@ __global__ void __launch_bounds__(kThreads, 8) flight_kernel(const __grid_consta
     constexpr int EPW = 32 / LPE;
     constexpr unsigned FULL = 0xffffffffu;
     constexpr unsigned GBITS = (LPE == 32) ? 0xffffffffu : ((1u << (LPE & 31)) - 1u);
-    extern __shared__ __align__(16) double smem[];
 
     const int tid = threadIdx.x, warp = tid >> 5, lane32 = tid & 31;
     const int wenv0 = (blockIdx.x * (kThreads / 32) + warp) * EPW;      // first env of this warp
     const int wcnt = min(EPW, p.E - wenv0);
     if (wcnt <= 0) return;                                               // whole warp idle (nothing is block-synchronised)
-    double* W = smem + (size_t)warp * p.s_warp;
-    longlong2* lutm = reinterpret_cast<longlong2*>(W + p.s_lut);
     const int n = p.n, m = p.m;
     const int g = lane32 / LPE, lane = lane32 % LPE, gbase = lane32 - lane;
     const bool active = g < wcnt;
@@ -56,14 +52,6 @@ __global__ void __launch_bounds__(kThreads, 8) flight_kernel(const __grid_consta
     if (active) {
         meta_ld(p, e, &m0, &m1);                                               // same addresses for the whole group
     }
-    if (MODE == MODE_STEP) {
-        const longlong2 v0 = __ldg(p.lut_meta + lane32);
-        longlong2 v1 = make_longlong2(0, 0);
-        if (lane32 + 32 < 37) v1 = __ldg(p.lut_meta + lane32 + 32);
-        lutm[lane32] = v0;
-        if (lane32 + 32 < 37) lutm[lane32 + 32] = v1;
-        __syncwarp();
-    }
     uint32_t found = m0.x, newf_last = m0.y, outmask = m0.z, time_step = m0.w;
     uint32_t episode = m1.x, flags = m1.y;
     float ep_reward = __uint_as_float(m1.z);
@@ -89,7 +77,7 @@ __global__ void __launch_bounds__(kThreads, 8) flight_kernel(const __grid_consta
             double h = yaw + ((act == 1) ? p.turn : ((act == 2) ? -p.turn : 0.0));   // dyaw = [0, pi/18, -pi/18] (:259-262)
             if (h > p.two_pi) h -= p.two_pi;                                          // strict tests (:263-266)
             else if (h < 0.0) h += p.two_pi;
-            { const double2 sc = heading_sincos(p, lutm, h); s_h = sc.x; c_h = sc.y; }
+            { const double2 sc = heading_sincos(p, h); s_h = sc.x; c_h = sc.y; }
             yaw = h;
         }
         // Can any repulsion term be non-zero this step?  If every pair of OLD positions is farther apart than
@@ -330,29 +318,20 @@ cudaError_t launch_flight(cs_flight* h, int mode, const uint8_t* actions, const 
                           cudaStream_t st) {
     if (h->p.variant) {
         if (mode == MODE_STEP)
-            flight_kernel<LPE, MODE_STEP, true><<<h->grid, kThreads, h->smem_bytes, st>>>(h->p, actions, mask, rflags, h->seq);
+            flight_kernel<LPE, MODE_STEP, true><<<h->grid, kThreads, 0, st>>>(h->p, actions, mask, rflags, h->seq);
         else
-            flight_kernel<LPE, MODE_RESET, true><<<h->grid, kThreads, h->smem_bytes, st>>>(h->p, actions, mask, rflags, h->seq);
+            flight_kernel<LPE, MODE_RESET, true><<<h->grid, kThreads, 0, st>>>(h->p, actions, mask, rflags, h->seq);
         // the belief maps of the envs the step / reset kernel just sensed (flight_env.py:266)
         const cudaError_t em = launch_map_generic(h, st);
         if (em != cudaSuccess) return em;
     } else {
         if (mode == MODE_STEP)
-            flight_kernel<LPE, MODE_STEP, false><<<h->grid, kThreads, h->smem_bytes, st>>>(h->p, actions, mask, rflags, 0u);
+            flight_kernel<LPE, MODE_STEP, false><<<h->grid, kThreads, 0, st>>>(h->p, actions, mask, rflags, 0u);
         else
-            flight_kernel<LPE, MODE_RESET, false><<<h->grid, kThreads, h->smem_bytes, st>>>(h->p, actions, mask, rflags, 0u);
+            flight_kernel<LPE, MODE_RESET, false><<<h->grid, kThreads, 0, st>>>(h->p, actions, mask, rflags, 0u);
     }
     cs_count_launch(1);
     return cudaGetLastError();
-}
-
-template <int LPE>
-cudaError_t set_smem_attr(size_t bytes) {
-    cudaError_t e = cudaFuncSetAttribute(flight_kernel<LPE, MODE_STEP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(flight_kernel<LPE, MODE_RESET, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(flight_kernel<LPE, MODE_STEP, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(flight_kernel<LPE, MODE_RESET, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    return e;
 }
 
 }  // namespace
@@ -366,23 +345,6 @@ cudaError_t launch_lpa(cs_flight* h, int mode, const uint8_t* actions, const uin
         case 16: return launch_flight<16>(h, mode, actions, mask, rflags, st);
         default: return launch_flight<32>(h, mode, actions, mask, rflags, st);
     }
-}
-
-// Dynamic shared memory limits are per KERNEL, not per handle: they are only ever raised, to the largest request any
-// handle of this process has made (a later, smaller handle must not lower them under an earlier one's launches).
-cudaError_t lpa_set_smem_limit(size_t step_bytes) {
-    static size_t cur_step = 48 * 1024;
-    cudaError_t e = cudaSuccess;
-    if (step_bytes > cur_step) {
-        e = set_smem_attr<1>(step_bytes);
-        if (e == cudaSuccess) e = set_smem_attr<2>(step_bytes);
-        if (e == cudaSuccess) e = set_smem_attr<4>(step_bytes);
-        if (e == cudaSuccess) e = set_smem_attr<8>(step_bytes);
-        if (e == cudaSuccess) e = set_smem_attr<16>(step_bytes);
-        if (e == cudaSuccess) e = set_smem_attr<32>(step_bytes);
-        if (e == cudaSuccess) cur_step = step_bytes;
-    }
-    return e;
 }
 
 }  // namespace csf

@@ -20,7 +20,8 @@ cudaError_t launch_map_generic(cs_flight* h, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-// per kernel, only ever raised (see lpa_set_smem_limit)
+// The dynamic shared memory limit is per KERNEL, not per handle: it is only ever raised, to the largest request any handle
+// of this process has made (a later, smaller handle must not lower it under an earlier one's launches).
 cudaError_t map_set_smem_limit(size_t generic_bytes) {
     static size_t cur = 48 * 1024;
     if (generic_bytes <= cur) return cudaSuccess;

@@ -36,48 +36,34 @@ namespace {
 #define CS_TPE_MIN_CTAS 8      // resident CTAs per SM the thread-per-env kernel is compiled for (register budget 65536/(64*N))
 #endif
 // One thread per env with the targets staged in shared memory (StagedView): up to three agents fit 10 CTAs per SM (102
-// registers) without spills when the sensing loop takes one target at a time -- measured on B200 (tools/sweep_stream.sh):
-// 1M envs 5.5e9 -> 6.2e9 env-steps/s, the grouped c2 launch 4.79e9 -> 4.83e9; with five agents the same setting spills
-// (65536 envs: 3.15e9 -> 2.78e9), so larger teams keep 8 CTAs and blocks of CS_TPE_TU targets.
+// registers) without spills when the sensing loop takes one target at a time -- measured on B200 with variant libraries
+// (tools/build_variant.sh): 1M envs 5.5e9 -> 6.2e9 env-steps/s, the grouped c2 launch 4.79e9 -> 4.83e9; with five agents
+// the same setting spills (65536 envs: 3.15e9 -> 2.78e9), so larger teams keep 8 CTAs and blocks of CS_TPE_TU targets.
 #ifndef CS_TPE_SMALL_CTAS
 #define CS_TPE_SMALL_CTAS 10
 #endif
 constexpr int tpe_min_ctas(int N, int K, int mode) { return (K == 1 && mode == 0 && N <= 3) ? CS_TPE_SMALL_CTAS : CS_TPE_MIN_CTAS; }
 
 // Where a thread finds its env's state.  GlobalView: straight from HBM, layout known at compile time (structure of arrays with
-// one thread per env, record per env otherwise).  TileView (flight_stream_kernel): the loads come from the shared-memory tile
-// that cp.async.bulk filled -- rows of kTileEnvs doubles: 3N agent rows, 4 meta rows, 2m target rows -- the stores go to HBM.
+// one thread per env, record per env otherwise).  StagedView (below): the same, with the target rows staged in shared memory.
 // What differs between the handles of a grouped launch comes from `g` (kernel parameter space), the rest from `p`.
-// streaming accesses of the state rows: evict-first, so that the heading table and the prefetched target rows stay in L1
-#ifdef CS_TPE_STREAM_HINTS
-__device__ __forceinline__ double ld_s(const double* q) { return __ldcs(q); }
-__device__ __forceinline__ uint2 ld_s(const uint2* q) { return __ldcs(q); }
-__device__ __forceinline__ void st_s(double* q, double v) { __stcs(q, v); }
-__device__ __forceinline__ void st_s(uint2* q, uint2 v) { __stcs(q, v); }
-#else
-__device__ __forceinline__ double ld_s(const double* q) { return *q; }
-__device__ __forceinline__ uint2 ld_s(const uint2* q) { return *q; }
-__device__ __forceinline__ void st_s(double* q, double v) { *q = v; }
-__device__ __forceinline__ void st_s(uint2* q, uint2 v) { *q = v; }
-#endif
-
 template <bool SOA>
 struct GlobalView {
-    static constexpr bool kTile = false, kStaged = false;
+    static constexpr bool kStaged = false;
     struct Ctx {};
     const FlightParams& p; const GroupEntry& g; int e;
     __device__ __forceinline__ GlobalView(const FlightParams& p_, const GroupEntry& g_, int e_, Ctx) : p(p_), g(g_), e(e_) {}
     __device__ __forceinline__ double* dynp(int row) const { return SOA ? g.dyn + (size_t)row * g.E + e : g.dyn + (size_t)e * p.rec + row; }
     __device__ __forceinline__ double2 xy_ld(int a) const {
-        if (SOA) { const double* q = dynp(2 * a); return make_double2(ld_s(q), ld_s(q + g.E)); }
+        if (SOA) { const double* q = dynp(2 * a); return make_double2(q[0], q[g.E]); }
         return *reinterpret_cast<const double2*>(dynp(2 * a));
     }
     __device__ __forceinline__ void xy_st(int a, double x, double y) const {
-        if (SOA) { double* q = dynp(2 * a); st_s(q, x); st_s(q + g.E, y); return; }
+        if (SOA) { double* q = dynp(2 * a); q[0] = x; q[g.E] = y; return; }
         *reinterpret_cast<double2*>(dynp(2 * a)) = make_double2(x, y);
     }
-    __device__ __forceinline__ double yaw_ld(int a) const { return SOA ? ld_s(dynp(p.yaw_off + a)) : *dynp(p.yaw_off + a); }
-    __device__ __forceinline__ void yaw_st(int a, double v) const { if (SOA) st_s(dynp(p.yaw_off + a), v); else *dynp(p.yaw_off + a) = v; }
+    __device__ __forceinline__ double yaw_ld(int a) const { return *dynp(p.yaw_off + a); }
+    __device__ __forceinline__ void yaw_st(int a, double v) const { *dynp(p.yaw_off + a) = v; }
     __device__ __forceinline__ double2 tgt_ld(int j) const {
         if (SOA) { const double* t = g.tgt + (size_t)(2 * j) * g.E + e; return make_double2(t[0], t[g.E]); }
         return *reinterpret_cast<const double2*>(g.tgt + ((size_t)e * p.m + j) * 2);
@@ -90,7 +76,7 @@ struct GlobalView {
     __device__ __forceinline__ void meta_ld(uint4* m0, uint4* m1) const {
         if (SOA) {
             const uint2* q = reinterpret_cast<const uint2*>(dynp(p.meta_off));
-            const uint2 a = ld_s(q), b = ld_s(q + g.E), c = ld_s(q + 2 * (size_t)g.E), d = ld_s(q + 3 * (size_t)g.E);
+            const uint2 a = q[0], b = q[g.E], c = q[2 * (size_t)g.E], d = q[3 * (size_t)g.E];
             *m0 = make_uint4(a.x, a.y, b.x, b.y);
             *m1 = make_uint4(c.x, c.y, d.x, d.y);
             return;
@@ -101,8 +87,8 @@ struct GlobalView {
     __device__ __forceinline__ void meta_st(uint4 m0, uint4 m1) const {
         if (SOA) {
             uint2* q = reinterpret_cast<uint2*>(dynp(p.meta_off));
-            st_s(q, make_uint2(m0.x, m0.y)); st_s(q + g.E, make_uint2(m0.z, m0.w));
-            st_s(q + 2 * (size_t)g.E, make_uint2(m1.x, m1.y)); st_s(q + 3 * (size_t)g.E, make_uint2(m1.z, m1.w));
+            q[0] = make_uint2(m0.x, m0.y); q[g.E] = make_uint2(m0.z, m0.w);
+            q[2 * (size_t)g.E] = make_uint2(m1.x, m1.y); q[3 * (size_t)g.E] = make_uint2(m1.z, m1.w);
             return;
         }
         uint4* mp = reinterpret_cast<uint4*>(dynp(p.meta_off));
@@ -158,41 +144,6 @@ struct StagedView : GlobalView<true> {
     __device__ __forceinline__ void targets_ready() const { asm volatile("cp.async.wait_all;" ::: "memory"); __syncwarp(); }
 };
 
-template <int N, int TE>
-struct TileView {
-    static constexpr bool kTile = true, kStaged = false;
-    struct Ctx { double* mine; };                 // this thread's column of the tile
-    const FlightParams& p; const GroupEntry& g; int e; double* mine;
-    static constexpr int kMetaRow = 3 * N, kTgtRow = 3 * N + 4;
-    __device__ __forceinline__ TileView(const FlightParams& p_, const GroupEntry& g_, int e_, Ctx c) : p(p_), g(g_), e(e_), mine(c.mine) {}
-    __device__ __forceinline__ double* dynp(int row) const { return g.dyn + (size_t)row * g.E + e; }
-    __device__ __forceinline__ double2 xy_ld(int a) const { return make_double2(mine[(2 * a) * TE], mine[(2 * a + 1) * TE]); }
-    __device__ __forceinline__ void xy_st(int a, double x, double y) const { double* q = dynp(2 * a); q[0] = x; q[g.E] = y; }
-    __device__ __forceinline__ double yaw_ld(int a) const { return mine[(2 * N + a) * TE]; }
-    __device__ __forceinline__ void yaw_st(int a, double v) const { *dynp(2 * N + a) = v; }
-    __device__ __forceinline__ double2 tgt_ld(int j) const { return make_double2(mine[(kTgtRow + 2 * j) * TE], mine[(kTgtRow + 2 * j + 1) * TE]); }
-    __device__ __forceinline__ void tgt_publish(int j, int es, int src, double2 v) const {
-        double* t = g.tgt + (size_t)(2 * j) * g.E + es;
-        t[0] = v.x; t[g.E] = v.y;
-        double* w = mine - (int)(threadIdx.x & 31) + src + (kTgtRow + 2 * j) * TE;        // the owner reads it back from the tile
-        w[0] = v.x; w[TE] = v.y;
-    }
-    __device__ __forceinline__ void meta_ld(uint4* m0, uint4* m1) const {
-        const uint2* q = reinterpret_cast<const uint2*>(mine + kMetaRow * TE);
-        const uint2 a = q[0], b = q[TE], c = q[2 * TE], d = q[3 * TE];
-        *m0 = make_uint4(a.x, a.y, b.x, b.y);
-        *m1 = make_uint4(c.x, c.y, d.x, d.y);
-    }
-    __device__ __forceinline__ void meta_st(uint4 m0, uint4 m1) const {
-        uint2* q = reinterpret_cast<uint2*>(dynp(p.meta_off));
-        q[0] = make_uint2(m0.x, m0.y); q[g.E] = make_uint2(m0.z, m0.w);
-        q[2 * (size_t)g.E] = make_uint2(m1.x, m1.y); q[3 * (size_t)g.E] = make_uint2(m1.z, m1.w);
-    }
-    template <int K>
-    __device__ __forceinline__ void prefetch_targets(int) const {}
-    __device__ __forceinline__ void targets_ready() const {}
-};
-
 __device__ __forceinline__ GroupEntry entry_of(const FlightParams& p) {
     GroupEntry g;
     g.E = p.E; g.env_id_base = p.env_id_base; g.seed = p.seed; g.pad = 0;
@@ -202,19 +153,10 @@ __device__ __forceinline__ GroupEntry entry_of(const FlightParams& p) {
     return g;
 }
 
-// heading-table index: 37 entries staged in shared memory once per CTA
-__device__ __forceinline__ void stage_lut_meta(const FlightParams& p, longlong2* lutm) {
-#ifdef CS_LUTM_STAGED
-    if (threadIdx.x < 37) lutm[threadIdx.x] = __ldg(p.lut_meta + threadIdx.x);
-    __syncthreads();
-#endif
-}
-
-// e_raw: the env of this thread (>= g.E: none); t_first: e_raw * K + kk of lane 0 of this warp; pre_act: for a TileView the
-// env's actions, 2 bits per agent, loaded one tile ahead by the caller.
+// e_raw: the env of this thread (>= g.E: none); t_first: e_raw * K + kk of lane 0 of this warp.
 template <int N, int K, int MODE, bool MAP, bool FUSED, class V>
-__device__ __forceinline__ int flight_tpe_body(const FlightParams& p, const GroupEntry& g, typename V::Ctx ctx, const longlong2* lutm,
-                                               const int e_raw, const int t_first, const uint8_t* __restrict__ actions, const uint32_t pre_act,
+__device__ __forceinline__ int flight_tpe_body(const FlightParams& p, const GroupEntry& g, typename V::Ctx ctx,
+                                               const int e_raw, const int t_first, const uint8_t* __restrict__ actions,
                                                const uint8_t* __restrict__ mask, uint32_t rflags, unsigned char* jobslots) {
     constexpr unsigned FULL = 0xffffffffu;
     static_assert(K == 1 || K == 4 || K == 8, "K");
@@ -258,7 +200,7 @@ __device__ __forceinline__ int flight_tpe_body(const FlightParams& p, const Grou
             for (int a = 0; a < N; ++a) {
                 int act;
                 if (actions != nullptr) {
-                    act = V::kTile ? (int)((pre_act >> (2 * a)) & 3u) : (int)actions[(size_t)e * N + a];
+                    act = (int)actions[(size_t)e * N + a];
                 } else {
                     // one Philox block serves 4 agents; action = word % 3 (np.random.randint(0, 3), agent.py:36)
                     if ((a & 3) == 0)
@@ -269,7 +211,7 @@ __device__ __forceinline__ int flight_tpe_body(const FlightParams& p, const Grou
                 double h = yaw[a] + ((act == 1) ? p.turn : ((act == 2) ? -p.turn : 0.0));   // dyaw = [0, pi/18, -pi/18] (:259-262)
                 if (h > p.two_pi) h -= p.two_pi;                                             // strict tests (:263-266)
                 else if (h < 0.0) h += p.two_pi;
-                const double2 sc = heading_sincos(p, lutm, h);
+                const double2 sc = heading_sincos(p, h);
                 s_h[a] = sc.x; c_h[a] = sc.y;
                 yaw[a] = h;
             }
@@ -548,8 +490,6 @@ __device__ __forceinline__ int flight_tpe_body(const FlightParams& p, const Grou
 template <int N, int K, int MODE, bool MAP>
 __global__ void __launch_bounds__(kTpeThreads, tpe_min_ctas(N, K, MAP ? 1 : MODE)) flight_tpe_kernel(const __grid_constant__ FlightParams p, const uint8_t* __restrict__ actions,
                                                                  const uint8_t* __restrict__ mask, uint32_t rflags) {
-    __shared__ longlong2 lutm[40];
-    if (MODE == MODE_STEP) stage_lut_meta(p, lutm);
     const GroupEntry g = entry_of(p);
     const int t0 = (int)blockIdx.x * kTpeThreads + (int)threadIdx.x;
     const int e_raw = t0 / K, t_first = t0 & ~31;
@@ -558,19 +498,19 @@ __global__ void __launch_bounds__(kTpeThreads, tpe_min_ctas(N, K, MAP ? 1 : MODE
         using S = StagedView<kTpeThreads>;
         typename S::Ctx ctx;
         ctx.col = tstage + threadIdx.x;
-        flight_tpe_body<N, K, MODE, false, false, S>(p, g, ctx, lutm, e_raw, t_first, actions, 0u, mask, rflags, nullptr);
+        flight_tpe_body<N, K, MODE, false, false, S>(p, g, ctx, e_raw, t_first, actions, mask, rflags, nullptr);
         return;
     }
     using V = GlobalView<K == 1>;                                       // one thread per env <-> structure of arrays (cs_flight_create)
     if (!MAP) {
-        flight_tpe_body<N, K, MODE, false, false, V>(p, g, typename V::Ctx{}, lutm, e_raw, t_first, actions, 0u, mask, rflags, nullptr);
+        flight_tpe_body<N, K, MODE, false, false, V>(p, g, typename V::Ctx{}, e_raw, t_first, actions, mask, rflags, nullptr);
         return;
     }
     // flight variant, two-kernel form: this env's belief-map job record for flight_map_tile_kernel, which runs next
     // (on the same stream, or on the handle's map stream): header {jobs, fill flag} + up to two job slots
     const int e = e_raw < p.E ? e_raw : p.E - 1;
     unsigned char* rec = p.jobs + (size_t)e * p.job_stride;
-    const int njobs = flight_tpe_body<N, K, MODE, true, false, V>(p, g, typename V::Ctx{}, lutm, e_raw, t_first, actions, 0u, mask, rflags, rec + 16);
+    const int njobs = flight_tpe_body<N, K, MODE, true, false, V>(p, g, typename V::Ctx{}, e_raw, t_first, actions, mask, rflags, rec + 16);
     if (e_raw < p.E && threadIdx.x % K == 0) {
         const int fill = (MODE == MODE_RESET && (rflags & CS_RESET_INIT) && (mask == nullptr || mask[e] != 0)) ? 1 : 0;   // reset(init=True): map <- 0.5 (flight_env.py:84-86)
         *reinterpret_cast<int2*>(rec) = make_int2(njobs, fill);
@@ -591,13 +531,11 @@ template <int N, int MODE>
 __global__ void __launch_bounds__(kFusedThreads, CS_FUSED_MIN_CTAS) flight_fused_kernel(const __grid_constant__ FlightParams p, const uint8_t* __restrict__ actions,
                                                                                        const uint8_t* __restrict__ mask, uint32_t rflags) {
     extern __shared__ __align__(16) unsigned char fsm[];
-    __shared__ longlong2 lutm[40];
-    if (MODE == MODE_STEP) stage_lut_meta(p, lutm);
     using V = GlobalView<false>;
     const GroupEntry g = entry_of(p);
     unsigned char* S = fsm + (size_t)(threadIdx.x / kFusedLanes) * p.fm_env;
     const int t0 = (int)blockIdx.x * kFusedThreads + (int)threadIdx.x;
-    const int njobs = flight_tpe_body<N, kFusedLanes, MODE, true, true, V>(p, g, typename V::Ctx{}, lutm, t0 / kFusedLanes, t0 & ~31, actions, 0u, mask,
+    const int njobs = flight_tpe_body<N, kFusedLanes, MODE, true, true, V>(p, g, typename V::Ctx{}, t0 / kFusedLanes, t0 & ~31, actions, mask,
                                                                             rflags, S + p.fm_job);
     const int e = min(t0 / kFusedLanes, p.E - 1);
     fused_map_phase<kFusedLanes>(p, e, (int)(threadIdx.x % kFusedLanes), S, njobs);
@@ -612,230 +550,19 @@ template <int N, int K>
 __global__ void __launch_bounds__(kTpeThreads, tpe_min_ctas(N, K, 0)) flight_tpe_group_kernel(const __grid_constant__ FlightParams common,
                                                                                        const __grid_constant__ GroupTable tab,
                                                                                        const __grid_constant__ GroupActions acts) {
-    __shared__ longlong2 lutm[40];
     const GroupEntry& g = tab.h[blockIdx.y];
     if ((long long)blockIdx.x * kTpeThreads >= (long long)g.E * K) return;          // handles may differ in num_envs
-    stage_lut_meta(common, lutm);
     const int t0 = (int)blockIdx.x * kTpeThreads + (int)threadIdx.x;
     if (K == 1) {
         extern __shared__ __align__(16) double tstage[];
         using S = StagedView<kTpeThreads>;
         typename S::Ctx ctx;
         ctx.col = tstage + threadIdx.x;
-        flight_tpe_body<N, K, MODE_STEP, false, false, S>(common, g, ctx, lutm, t0, t0 & ~31, acts.a[blockIdx.y], 0u, nullptr, 0u, nullptr);
+        flight_tpe_body<N, K, MODE_STEP, false, false, S>(common, g, ctx, t0, t0 & ~31, acts.a[blockIdx.y], nullptr, 0u, nullptr);
         return;
     }
     using V = GlobalView<false>;
-    flight_tpe_body<N, K, MODE_STEP, false, false, V>(common, g, typename V::Ctx{}, lutm, t0 / K, t0 & ~31, acts.a[blockIdx.y], 0u, nullptr, 0u, nullptr);
-}
-
-// ------------------------------------------------------------------------------------------------
-// The STREAMING step kernel (flight_easy, one thread per env, structure-of-arrays state; the default from 32768 envs per
-// launch and for grouped launches).  flight_tpe_kernel is bound by memory latency: every warp loads its 3N + 4 + 2m state
-// rows, waits, computes, stores.  Here the loads are taken off the warps.  One persistent CTA per SM walks over tiles of
-// kTileEnvs = 64 consecutive envs of one handle; the state rows of a tile (3N agent rows, 4 meta rows, 2m target rows of
-// 512 bytes, each contiguous in the structure-of-arrays layout) are brought into a slot of a shared-memory RING by
-// cp.async.bulk [SASS UBLKCP] completing on the slot's mbarrier.  The CTA's warps form `groups` of two; group g computes the
-// CTA's tiles g, g + groups, ... straight from shared memory while the tiles of the other ring slots (slots > groups) are
-// in flight.  A slot is refilled with the tile `slots` ahead by the LAST warp that finishes with it (a shared-memory
-// counter), so no warp ever waits for another one.  Stores go from registers to HBM (coalesced rows); the actions of a
-// group's next tile are loaded one tile ahead.  The arithmetic is flight_tpe_body's: bit-identical to the other kernels.
-// Needs an even num_envs (16-byte granularity of the bulk copies); other handles keep flight_tpe_kernel.
-// ------------------------------------------------------------------------------------------------
-#ifndef CS_STREAM_MAX_GROUPS
-#define CS_STREAM_MAX_GROUPS 6        // register budget: 65536 / (64 * groups) per thread
-#endif
-constexpr int kStreamWarps = 2, kTileEnvs = 32 * kStreamWarps;            // per group
-constexpr int kStreamMaxGroups = CS_STREAM_MAX_GROUPS, kStreamMaxSlots = 16;
-
-struct StreamGeom {
-    int tph;                 // tiles per handle (the largest handle's)
-    int total;               // tph * handles
-    int groups, slots;
-    int rows;                // 3N + 4 + 2m
-    uint32_t slot_bytes;     // rows * kTileEnvs * 8
-};
-
-template <int G> struct GroupTableT { GroupEntry h[G]; };
-template <int G> struct GroupActionsT { const uint8_t* a[G]; };
-
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(bar), "r"(parity) : "memory");
-}
-
-__device__ __forceinline__ void bulk_row(uint32_t dst, const double* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
-// one lane: start the bulk copies of tile (g, e0) into a ring slot; a tile beyond its handle's envs only completes the phase
-template <int N>
-__device__ __forceinline__ void stream_issue(const FlightParams& common, const GroupEntry& g, const int e0, const uint32_t dst, const uint32_t bar) {
-    if (e0 >= g.E) {
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-        return;
-    }
-    const int cnt = min(kTileEnvs, g.E - e0);
-    const uint32_t bytes = (uint32_t)cnt * 8u;
-    const int rows_t = 2 * common.m;
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes * (uint32_t)(3 * N + 4 + rows_t)) : "memory");
-    const size_t E = (size_t)g.E;
-    const double* src = g.dyn + e0;
-    uint32_t d = dst;
-#pragma unroll
-    for (int r = 0; r < 3 * N; ++r, d += kTileEnvs * 8, src += E) bulk_row(d, src, bytes, bar);
-    src = g.dyn + (size_t)common.meta_off * E + e0;
-#pragma unroll
-    for (int r = 0; r < 4; ++r, d += kTileEnvs * 8, src += E) bulk_row(d, src, bytes, bar);
-    src = g.tgt + e0;
-#pragma unroll 6
-    for (int r = 0; r < rows_t; ++r, d += kTileEnvs * 8, src += E) bulk_row(d, src, bytes, bar);
-}
-
-template <int N, int G>
-__global__ void __launch_bounds__(kTileEnvs * kStreamMaxGroups, 1) flight_stream_kernel(const __grid_constant__ FlightParams common,
-                                                                                       const __grid_constant__ GroupTableT<G> tab,
-                                                                                       const __grid_constant__ GroupActionsT<G> acts,
-                                                                                       const __grid_constant__ StreamGeom geo) {
-    extern __shared__ __align__(128) unsigned char ssm[];
-    __shared__ longlong2 lutm[40];
-    __shared__ __align__(8) uint64_t full[kStreamMaxSlots];
-    __shared__ int drained[kStreamMaxSlots];
-    // fills started per slot.  A parity wait alone cannot tell "fill u has not landed" from "fill u - 1 has not even been
-    // started" (a group may get to tile q before another group has drained tile q - 2 * slots); the count can.
-    __shared__ volatile int issued[kStreamMaxSlots];
-    const int tid = threadIdx.x, lane = tid & 31, grp = tid / kTileEnvs, gt = tid % kTileEnvs;
-    const int R = geo.slots, GR = geo.groups, step = (int)gridDim.x;
-    // tile q of this CTA (q = 0, 1, ...) is global tile blockIdx.x + q * gridDim.x and lives in ring slot q % R
-    const int nq = (geo.total - (int)blockIdx.x + step - 1) / step;
-    auto tile_of = [&](int q, int* h, int* e0) {
-        const int t = (int)blockIdx.x + q * step;
-        *h = t / geo.tph;
-        *e0 = (t - *h * geo.tph) * kTileEnvs;
-    };
-    if (tid == 0) {
-        for (int s = 0; s < R; ++s) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(full + s)));
-            drained[s] = 0;
-            issued[s] = s < nq ? 1 : 0;
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    stage_lut_meta(common, lutm);                       // (block-wide barrier: the mbarriers are visible too)
-    if (tid == 0) {                                     // prologue: fill the ring
-        for (int q = 0; q < R && q < nq; ++q) {
-            int h, e0;
-            tile_of(q, &h, &e0);
-            stream_issue<N>(common, tab.h[h], e0, smem_u32(ssm + (size_t)q * geo.slot_bytes), smem_u32(full + q));
-        }
-    }
-    // raw action bytes of this thread's env in the group's next tile: loaded one tile ahead, consumed at the top of the loop
-    uint32_t raw[N];
-    auto load_actions = [&](int q) {
-#pragma unroll
-        for (int k = 0; k < N; ++k) raw[k] = 0u;
-        if (q < nq) {
-            int h, e0;
-            tile_of(q, &h, &e0);
-            const uint8_t* a = acts.a[h];
-            if (a != nullptr && e0 + gt < tab.h[h].E) {
-                a += (size_t)(e0 + gt) * N;
-#pragma unroll
-                for (int k = 0; k < N; ++k) raw[k] = a[k];
-            }
-        }
-    };
-    load_actions(grp);
-    int slot = grp % R, use = grp / R;                  // ring position of tile q, maintained incrementally
-    for (int q = grp; q < nq; q += GR) {
-        int h, e0;
-        tile_of(q, &h, &e0);
-        const GroupEntry& g = tab.h[h];
-        uint32_t act_cur = 0;
-#pragma unroll
-        for (int k = 0; k < N; ++k) act_cur |= (raw[k] & 3u) << (2 * k);
-        load_actions(q + GR);
-        while (issued[slot] <= use) __nanosleep(64);
-        mbar_wait(smem_u32(full + slot), (uint32_t)use & 1u);
-        if (e0 < g.E) {                                 // (handles may differ in num_envs)
-            using V = TileView<N, kTileEnvs>;
-            typename V::Ctx ctx;
-            ctx.mine = reinterpret_cast<double*>(ssm + (size_t)slot * geo.slot_bytes) + gt;
-            flight_tpe_body<N, 1, MODE_STEP, false, false, V>(common, g, ctx, lutm, e0 + gt, e0 + (gt & ~31), acts.a[h], act_cur, nullptr, 0u, nullptr);
-        }
-        // this warp is done with the slot; the last warp of the group to get here refills it with the tile `slots` ahead
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) {
-            __threadfence_block();
-            const int old = atomicAdd(&drained[slot], 1);
-            if (old == kStreamWarps - 1) {
-                drained[slot] = 0;
-                __threadfence_block();
-                if (q + R < nq) {
-                    int hn, en;
-                    tile_of(q + R, &hn, &en);
-                    stream_issue<N>(common, tab.h[hn], en, smem_u32(ssm + (size_t)slot * geo.slot_bytes), smem_u32(full + slot));
-                    __threadfence_block();
-                    issued[slot] = use + 2;
-                }
-            }
-        }
-        slot += GR;
-        while (slot >= R) { slot -= R; ++use; }
-    }
-}
-
-template <int N, int G>
-cudaError_t launch_stream(const FlightParams& common, const GroupTableT<G>& tab, const GroupActionsT<G>& acts, int count, int max_E, cudaStream_t st) {
-    static int sm_count = 0, max_smem = 0;
-    static size_t smem_set = 0;
-    if (sm_count == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-        cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-    }
-    StreamGeom geo;
-    geo.rows = 3 * N + 4 + 2 * common.m;
-    geo.slot_bytes = (uint32_t)geo.rows * kTileEnvs * 8u;
-    geo.tph = (max_E + kTileEnvs - 1) / kTileEnvs;
-    geo.total = geo.tph * count;
-    int groups = kStreamMaxGroups, slots = 0;
-    if (const char* v = getenv("CS_STREAM_GROUPS")) groups = atoi(v);               // tuning sweeps
-    if (const char* v = getenv("CS_STREAM_SLOTS")) slots = atoi(v);
-    groups = groups < 1 ? 1 : (groups > kStreamMaxGroups ? kStreamMaxGroups : groups);
-    const int fit = (int)(((size_t)max_smem - 1024) / geo.slot_bytes);
-    if (slots < 1 || slots > fit) slots = fit;
-    if (slots > kStreamMaxSlots) slots = kStreamMaxSlots;
-    if (slots < 2) return cudaErrorInvalidConfiguration;
-    if (groups > slots - 1) groups = slots - 1;                 // at least one tile in flight
-    geo.groups = groups; geo.slots = slots;
-    const size_t smem = (size_t)slots * geo.slot_bytes;
-    auto kern = flight_stream_kernel<N, G>;
-    if (smem > smem_set) {                                        // only ever raised (other handles may need more)
-        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        smem_set = smem;
-    }
-    int grid = geo.total < sm_count ? geo.total : sm_count;
-    if (const char* v = getenv("CS_STREAM_GRID")) { const int gv = atoi(v); if (gv >= 1 && gv < grid) grid = gv; }   // tests: many tiles per CTA on small handles
-    kern<<<grid, kTileEnvs * groups, smem, st>>>(common, tab, acts, geo);
-    cs_count_launch(1);
-    return cudaGetLastError();
-}
-
-// opt-in (CS_STREAM=1): measured slower than flight_tpe_kernel on B200 (DESIGN.md section 4.2), kept for the record
-inline bool stream_enabled() {
-    const char* v = getenv("CS_STREAM");
-    return v && atoi(v) == 1;
+    flight_tpe_body<N, K, MODE_STEP, false, false, V>(common, g, typename V::Ctx{}, t0 / K, t0 & ~31, acts.a[blockIdx.y], nullptr, 0u, nullptr);
 }
 
 // shared-memory staging area of the targets in the one-thread-per-env step kernels: 2m rows of kTpeThreads doubles
@@ -843,17 +570,6 @@ inline size_t tstage_bytes(int m) { return (size_t)2 * m * kTpeThreads * sizeof(
 
 template <int N, int K>
 cudaError_t launch_tpe_k(cs_flight* h, int mode, const uint8_t* actions, const uint8_t* mask, uint32_t rflags, cudaStream_t st) {
-    if (K == 1 && mode == MODE_STEP && !h->p.variant && h->p.E % 2 == 0 && stream_enabled()) {
-        GroupTableT<1> tab;
-        GroupActionsT<1> acts;
-        const FlightParams& p = h->p;
-        GroupEntry& t = tab.h[0];
-        t.E = p.E; t.env_id_base = p.env_id_base; t.seed = p.seed; t.pad = 0; t.dyn_rs = p.dyn_rs; t.dyn_es = p.dyn_es; t.tgt_rs = p.tgt_rs; t.tgt_es = p.tgt_es;
-        t.dyn = p.dyn; t.tgt = p.tgt; t.obs = p.obs; t.state = p.state; t.reward = p.reward; t.terminated = p.terminated; t.win = p.win;
-        t.target_find = p.target_find; t.stats = p.stats; t.tmpl = p.tmpl;
-        acts.a[0] = actions;
-        return launch_stream<N, 1>(p, tab, acts, 1, p.E, st);
-    }
     const long long threads = (long long)h->p.E * K;
     const int grid = (int)((threads + kTpeThreads - 1) / kTpeThreads);
     if (h->p.variant) {
@@ -895,11 +611,6 @@ cudaError_t launch_tpe_n(cs_flight* h, int mode, const uint8_t* actions, const u
 
 template <int N>
 cudaError_t launch_group_n(const cs_flight_group* g, const GroupActions& acts, cudaStream_t st) {
-    if (g->k == 1 && g->all_even && stream_enabled()) {
-        static_assert(sizeof(GroupTableT<kMaxGroup>) == sizeof(GroupTable) && sizeof(GroupActionsT<kMaxGroup>) == sizeof(GroupActions), "table layout");
-        return launch_stream<N, kMaxGroup>(g->envs[0]->p, reinterpret_cast<const GroupTableT<kMaxGroup>&>(g->table),
-                                           reinterpret_cast<const GroupActionsT<kMaxGroup>&>(acts), g->count, g->max_E, st);
-    }
     const dim3 grid((unsigned)g->grid_x, (unsigned)g->count);
     if (g->k == 1) flight_tpe_group_kernel<N, 1><<<grid, kTpeThreads, tstage_bytes(g->envs[0]->p.m), st>>>(g->envs[0]->p, g->table, acts);
     else flight_tpe_group_kernel<N, 4><<<grid, kTpeThreads, 0, st>>>(g->envs[0]->p, g->table, acts);

@@ -153,24 +153,13 @@ def test_thread_per_env_kernel_equals_lane_per_agent_kernel(n_agents, agent_mode
 
 
 @pytest.mark.parametrize("n_agents,agent_mode,target_mode,time_limit,E",
-                         [(3, 0, 0, 40, 1000), (3, 0, 0, 12, 2), (5, 2, 1, 30, 130), (8, 3, 1, 25, 4222), (1, 1, 0, 20, 258), (4, 0, 0, 15, 640)])
-def test_streaming_step_kernel_equals_lane_per_agent_kernel(monkeypatch, n_agents, agent_mode, target_mode, time_limit, E):
-    """flight_stream_kernel (opt-in with CS_STREAM=1: persistent CTAs, state tiles staged in shared memory by cp.async.bulk;
-    lanes_per_env = 1 and an even num_envs) against flight_kernel, bit for bit: partial tiles, one and many tiles per CTA,
-    auto-resets whose redrawn targets are read back from the tile, device actions and the in-kernel random policy."""
-    monkeypatch.setenv("CS_STREAM", "1")
+                         [(3, 0, 0, 40, 1000), (3, 0, 0, 12, 2), (5, 2, 1, 30, 130), (8, 3, 1, 25, 4222), (1, 1, 0, 20, 258), (4, 0, 0, 15, 640),
+                          (3, 0, 0, 12, 40000)])
+def test_one_thread_per_env_kernel_shapes_equal_lane_per_agent_kernel(n_agents, agent_mode, target_mode, time_limit, E):
+    """flight_tpe_kernel<N, 1> (lanes_per_env = 1: one thread per env, structure-of-arrays state, targets staged in shared
+    memory) against flight_kernel, bit for bit: partial warps and CTAs, a single agent, eight agents, and auto-resets whose
+    redrawn targets are read back from the staging area, under device actions and the in-kernel random policy."""
     compare_step_kernels(n_agents, agent_mode, target_mode, 50, time_limit, "easy", E, 1)
-
-
-@pytest.mark.parametrize("groups,slots,grid", [(2, 3, 3), (6, 7, 1), (1, 2, 2), (5, 10, 2), (6, 10, 148)])
-def test_streaming_step_kernel_ring_reuse(monkeypatch, groups, slots, grid):
-    """The same comparison with few CTAs and a short ring, so that every ring slot is refilled many times and the warp
-    groups of a CTA run far apart (the tuning variables are read at every launch)."""
-    monkeypatch.setenv("CS_STREAM", "1")
-    monkeypatch.setenv("CS_STREAM_GROUPS", str(groups))
-    monkeypatch.setenv("CS_STREAM_SLOTS", str(slots))
-    monkeypatch.setenv("CS_STREAM_GRID", str(grid))
-    compare_step_kernels(3, 0, 0, 50, 12, "easy", 4222 if grid < 148 else 40000, 1)
 
 
 @pytest.mark.parametrize("variant,n_agents", [("probmap", 3), ("easy", 5), ("probmap", 6)])
@@ -410,15 +399,13 @@ def test_pooled_host_stepper_reset_list_tail_and_overflow():
     assert any(85 < c <= 256 for c in resets_seen) and any(c > 256 for c in resets_seen), resets_seen
 
 
-@pytest.mark.parametrize("lpe,sizes", [(1, [700, 4096, 33]), (1, [700, 4096, 34, 2, 128]), (-1, [700, 4096, 34, 2, 128]), (4, [256, 256, 256, 1000]), (0, [512, 512])])
-def test_grouped_device_step_equals_separate_steps(monkeypatch, lpe, sizes):
+@pytest.mark.parametrize("lpe,sizes", [(1, [700, 4096, 33]), (1, [700, 4096, 34, 2, 128]), (4, [700, 4096, 34, 2, 128]), (4, [256, 256, 256, 1000]), (0, [512, 512])])
+def test_grouped_device_step_equals_separate_steps(lpe, sizes):
     """cs_flight_group_step: env batches of different sizes stepped in ONE launch end up bit-identical to the same
     batches stepped one by one (state, targets, outputs, statistics), through episode ends and in-call auto-resets."""
     import coopsearch_b200 as cs
     spec = FlightSpec(n_agents=3, time_limit=20)
     args = make_args(dict(spec.__dict__))
-    stream_group = lpe == -1           # the grouped launch through the streaming kernel, the separate steps through flight_tpe_kernel
-    lpe = 1 if stream_group else lpe
     mk = lambda: [cs.VecFlightEasyEnv(args, TEMPLATE, num_envs=E, seed=9, env_id_base=1000 * b, auto_reset=True, lanes_per_env=lpe)
                   for b, E in enumerate(sizes)]
     ref, envs = mk(), mk()
@@ -426,10 +413,7 @@ def test_grouped_device_step_equals_separate_steps(monkeypatch, lpe, sizes):
     gen = torch.Generator(device="cuda").manual_seed(3)
     for t in range(50):
         acts = [torch.randint(0, 3, (E, 3), dtype=torch.uint8, device="cuda", generator=gen) for E in sizes]
-        if stream_group:
-            monkeypatch.setenv("CS_STREAM", "1")
         stepper.step(acts)
-        monkeypatch.delenv("CS_STREAM", raising=False)
         for a, e, r in zip(acts, envs, ref):
             rr, rt, rw = r.step(a)
             assert torch.equal(rr, e._reward) and torch.equal(rt, e._terminated) and torch.equal(rw, e._win), "step %d" % t

@@ -3,9 +3,8 @@
 mkdir -p gpurun_out/r2
 out=gpurun_out/r2/sanitizer_r02.txt
 : > $out
-for mode in "memcheck 0" "memcheck 1" "racecheck 0"; do
-  set -- $mode
-  echo "== compute-sanitizer --tool $1 (CS_STREAM=$2)" >> $out
-  CS_STREAM=$2 timeout 900 compute-sanitizer --tool $1 python tools/sanitize_run.py 2>&1 | grep -E "sanitize_run done|ERROR SUMMARY|RACECHECK SUMMARY|Invalid|hazard|Error" | head -12 >> $out
+for tool in memcheck racecheck; do
+  echo "== compute-sanitizer --tool $tool" >> $out
+  timeout 900 compute-sanitizer --tool $tool python tools/sanitize_run.py 2>&1 | grep -E "sanitize_run done|ERROR SUMMARY|RACECHECK SUMMARY|Invalid|hazard|Error" | head -12 >> $out
 done
 cat $out

@@ -10,13 +10,12 @@ def fargs(n, M=50, R=7, T=25, am=0):
     return types.SimpleNamespace(env="x", map_size=M, target_num=15, target_mode=0, agent_mode=am, n_agents=n, view_range=R,
                                  time_limit=T, detect_prob=0.9, safe_dist=1, agent_velocity=1, force_dist=3)
 # (class, agents, map size, lanes_per_env: 0 = thread-per-env kernel (flight variant: fused step + map kernel),
-#  16 = lane-per-agent kernel (+ generic map kernel))
+#  16 = lane-per-agent kernel (+ generic map kernel)); CS_SAN_K=1 or 4 replaces the automatic choice (0)
+san_k = int(os.environ.get("CS_SAN_K", "0"))
 for cls, n, M, lpe in ((cs.VecFlightEasyEnv, 3, 50, 0), (cs.VecFlightEasyEnv, 5, 12, 0), (cs.VecFlightEasyEnv, 3, 50, 16),
                        (cs.VecFlightEnv, 3, 50, 0), (cs.VecFlightEnv, 8, 63, 0), (cs.VecFlightEnv, 5, 50, 16),
                        (cs.VecFlightEnv, 2, 51, 0), (cs.VecFlightEnv, 2, 70, 0)):
-    if os.environ.get("CS_SAN_K"):
-        os.environ["CS_TPE_K"] = os.environ["CS_SAN_K"]
-    env = cls(fargs(n, M=M, R=min(7, M // 3)), gu.TEMPLATE, num_envs=37, seed=1, auto_reset=True, count_touched=True, lanes_per_env=lpe)
+    env = cls(fargs(n, M=M, R=min(7, M // 3)), gu.TEMPLATE, num_envs=37, seed=1, auto_reset=True, count_touched=True, lanes_per_env=lpe or san_k)
     env.step_random(40)
     acts = torch.randint(0, 3, (37, n), dtype=torch.uint8, device="cuda")
     env.step(acts)
@@ -26,7 +25,7 @@ for cls, n, M, lpe in ((cs.VecFlightEasyEnv, 3, 50, 0), (cs.VecFlightEasyEnv, 5,
         env.set_obs_kernel("plain"); env.get_obs()
         env.prob_map = env.prob_map
     env.stats()
-# round 2: one thread per env with staged targets (lanes_per_env=1; 38 envs = even, so CS_STREAM=1 takes the streaming kernel),
+# round 2: one thread per env with staged targets (lanes_per_env=1),
 # the grouped launch, the pooled host path (pack kernel, strided copy), the episode writer, the agent network on the tensor
 # cores with the conv front end, simple_spread
 for n in (3, 5):

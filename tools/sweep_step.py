@@ -1,4 +1,4 @@
-"""Step kernel sweep: python tools/sweep_step.py [workloads...]; env CS_TPE_K / CS_BENCH_LPE / CS_BENCH_STREAMS select the variant."""
+"""Step kernel sweep: python tools/sweep_step.py [workloads...]; env CS_BENCH_LPE / CS_BENCH_STREAMS select the variant."""
 import os
 import sys
 
@@ -11,7 +11,7 @@ import coopsearch_b200 as cs  # noqa: E402
 dev = torch.device("cuda", 0)
 torch.cuda.set_device(dev)
 names = sys.argv[1:] or ["c2", "c3", "c2w"]
-tag = "K=%s LPE=%s streams=%s" % (os.environ.get("CS_TPE_K", "-"), os.environ.get("CS_BENCH_LPE", "0"), os.environ.get("CS_BENCH_STREAMS", "8"))
+tag = "LPE=%s streams=%s" % (os.environ.get("CS_BENCH_LPE", "0"), os.environ.get("CS_BENCH_STREAMS", "8"))
 for name in names:
     steps = {"c2": 60, "c2s": 60, "c3": 100, "c2w": 30, "c4": 100}.get(name, 50)
     r = bench.run_gpu_workload(cs, torch, name, steps, 5, dev, 0, 1, want_e2e=(name in ("c2", "c2s")), burn_in_s=0.2)
